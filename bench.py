@@ -172,6 +172,24 @@ def measured_peaks():
         return None
 
 
+def oracle_built():
+    from oracle import oracle_py
+    return oracle_py.available("native") or oracle_py.available("parity")
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Each array as float32 DIR/<name>.npy.  Past DUMP_LIMIT bytes in all, every s-th element of each (flattened) array is kept instead, the same
+    elements on every run, so that two builds can still be compared output for output."""
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    stride = -(-sum(a.nbytes for a in arrays.values()) // DUMP_LIMIT)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a if stride == 1 else np.ascontiguousarray(a.reshape(-1)[::stride]))
+
+
 def bvh_bytes(nodes, tris):
     """SURVEY.md 8(d): 64 B per BVH node visited + 48 B per triangle tested."""
     return 64 * nodes + 48 * tris
@@ -344,6 +362,7 @@ def main():
     ap.add_argument("--no-split-leftover", action="store_true", help="iteration mode: deal the K %% N left-over iterations whole instead of splitting each by camera tile over N / (K %% N) ranks (A/B switch)")
     ap.add_argument("--no-path-tracer", action="store_true", help="skip the extra `path_tracer` key (the second device integrator on the same workload, N = 1 only)")
     ap.add_argument("--cpu-budget", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed (the Result film after its last step) to DIR/<name>.npy")
     ap.add_argument("--lanes", type=int, default=4, help="iterations in flight per GPU (etxb_group); 1 = the plain one-context pump")
     ap.add_argument("--parallelism", default="both", choices=["both", "tile", "iteration"],
                     help="N > 1: how the job's K iterations are spread over the GPUs.  'tile' (the north star's mode) = every iteration split by pixel tile "
@@ -488,7 +507,7 @@ def main():
         light_vertices = st1["light_vertices"]
         g.close()
         return {"mode": mode, "value": n_pixels * args.steps / elapsed / 1e6, "elapsed": elapsed, "counters": counters, "clocks": clk,
-                "lanes": mode_lanes,
+                "lanes": mode_lanes, "film": host_film.copy() if (args.dump_outputs and rank == 0) else None,
                 "e2e": {"value": n_pixels * args.steps / e2e_s / 1e6, "unit": UNIT, "h2d_bytes_per_step": int(g.options.nbytes) * mode_lanes,
                         "d2h_bytes_per_step": int(host_film.nbytes * film_reads / args.steps)},
                 "collective_ms_per_iteration": comm_ms or None, "film_finite": finite, "light_vertices": light_vertices}
@@ -601,13 +620,15 @@ def main():
                             "`traffic` = ncu dram read+write of one head-of-pass launch of the kernel (profiles/ncu_traffic.json).  The photon gather is served from L2 "
                             "(82 % hit rate) and the bounce kernels are latency / FP32 bound, so these fractions of the HBM copy peak are not DRAM utilisation"}
         cpu = None
-        if not args.no_cpu_baseline:
+        if not args.no_cpu_baseline and not oracle_built():
+            cpu = {"unavailable": "oracle/_ref is not built (build() makes it where the reference sources exist)"}
+        elif not args.no_cpu_baseline:
             from etx_tracer_b200 import scenes
             cpu, _ = cpu_baseline_run(lambda res: scene_factory(args, res), args.cpu_budget, os.cpu_count() or 1, workload_vcm_options(args))
         pt = None
         if (world == 1) and not args.no_path_tracer:
             try:
-                pt = path_tracer_line(sd, local_rank, cpu_iterations=0 if args.no_cpu_baseline else 1)
+                pt = path_tracer_line(sd, local_rank, cpu_iterations=0 if (args.no_cpu_baseline or not oracle_built()) else 1)
             except Exception as e:  # an extra key must never cost the headline line
                 pt = {"error": f"{type(e).__name__}: {e}"[:300]}
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -632,6 +653,8 @@ def main():
                 # every way of spreading the same K iterations that was measured in this run (N > 1, --parallelism both): `value` is the faster one
                 "modes": {r["mode"]: {"value": r["value"], "ms_per_step": r["elapsed"] / args.steps * 1e3, "e2e": r["e2e"]["value"],
                                       "collective_ms_per_iteration": r["collective_ms_per_iteration"], "film_finite": r["film_finite"]} for r in results}}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"film_result": best["film"]})
         if json_fd is not None:
             sys.stdout.flush()
             os.write(json_fd, (json.dumps(line) + "\n").encode())

@@ -11,7 +11,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, bit_equal, golden, rel_l2
+from conftest import GOLDEN, Digest, bit_equal, golden, rel_l2, same_bits
 from etx_tracer_b200 import scenes, structs as S
 
 pytestmark = pytest.mark.gpu
@@ -51,30 +51,40 @@ def _device(api, sd, iterations, options=None, settings=None, flavor="parity", f
     return g
 
 
-def _assert_bit_exact(g, o, what=""):
-    for bid, dt in ((S.BUF_CAMERA_SAMPLER, np.uint32), (S.BUF_CAMERA_GATHERED, np.float32), (S.BUF_PIXEL_INFO, np.uint32)):
-        a, b = g.buffer(bid, dt), o.buffer(bid, dt)
-        assert a.shape == b.shape, f"{what} buffer {bid}: {a.shape} vs {b.shape}"
-        same = a.view(np.uint32) == b.view(np.uint32)
-        assert same.all(), f"{what} buffer {bid}: {100.0 * same.mean():.3f}% identical, first mismatch at {int(np.argmin(same))}"
-    for layer in LAYERS:
-        a, b = g.film(layer)[..., :3], o.film(layer)[..., :3]
-        same = a.view(np.uint32) == b.view(np.uint32)
-        assert same.all(), f"{what} film layer {layer}: {100.0 * same.mean():.3f}% identical"
-    assert g.pt_status()["pixels_processed"] == o.pt_status()["pixels_processed"]
+PT_BUFFERS = ((S.BUF_CAMERA_SAMPLER, np.uint32), (S.BUF_CAMERA_GATHERED, np.float32), (S.BUF_PIXEL_INFO, np.uint32))
 
 
-def _compare(api, oracle_mod, sd, iterations, options=None, settings=None, what=""):
-    o = _oracle(oracle_mod, sd, iterations, options, settings)
-    g = _device(api, sd, iterations, options, settings)
-    _assert_bit_exact(g, o, what)
-    gc, oc = g.counters(), o.counters()
+def _outputs(x, sd):
+    """What the parity tests compare, of a device context or an oracle: the counters come as a dict from the one, a record from the other."""
+    out = {f"buffer {bid}": x.buffer(bid, dt) for bid, dt in PT_BUFFERS}
+    out.update({f"film layer {layer}": x.film(layer)[..., :3] for layer in LAYERS})
+    out["pixels_processed"] = x.pt_status()["pixels_processed"]
+    c = x.counters()
     # one shaded event per run_path_iteration call that got past the length test; closest-hit queries likewise unless a subsurface walk adds its own
-    assert gc["bounces_camera"] == int(oc["bounces_camera"][0]), what
+    out["bounces_camera"] = int(np.asarray(c["bounces_camera"]).reshape(-1)[0])
     if int(sd.scene["subsurface_scatter_material"][0]) == S.INVALID:
-        assert gc["rays_closest"] == int(oc["rays_closest"][0]), what
+        out["rays_closest"] = int(np.asarray(c["rays_closest"]).reshape(-1)[0])
+    return out
+
+
+def _assert_bit_exact(got, ref, what=""):
+    assert sorted(got) == sorted(ref), what
+    for k in ref:
+        a, b = got[k], ref[k]
+        if isinstance(b, Digest):
+            assert same_bits(a, b), f"{what} {k} differs from the oracle's"
+            continue
+        a, b = np.asarray(a), np.asarray(b)
+        assert a.shape == b.shape, f"{what} {k}: {a.shape} vs {b.shape}"
+        same = a.view(np.uint32) == b.view(np.uint32) if a.dtype.itemsize == 4 else a == b
+        assert same.all(), f"{what} {k}: {100.0 * same.mean():.3f}% identical, first mismatch at {int(np.argmin(same))}"
+
+
+def _compare(api, oracle_record, sd, iterations, options=None, settings=None, what=""):
+    ref = oracle_record(what, lambda m: _outputs(_oracle(m, sd, iterations, options, settings), sd))
+    g = _device(api, sd, iterations, options, settings)
+    _assert_bit_exact(_outputs(g, sd), ref, what)
     g.close()
-    o.close()
 
 
 C1 = dict(samples=16, spectral=False)
@@ -100,9 +110,9 @@ def test_path_tracer_matches_committed_golden_render(api):
     (C1, dict(direct=0), None),                # light sampling only
     (C2, None, (0.0, 0.5)),                    # radiance clamp (path_tracing.cxx:73-78)
 ])
-def test_iterations_are_bit_exact_against_live_oracle(api, oracle_mod, kwargs, options, settings):
+def test_iterations_are_bit_exact_against_live_oracle(api, oracle_record, kwargs, options, settings):
     sd = scenes.cornell_box(48, 40, **kwargs)  # non-square film exercises the y-flip and aspect handling
-    _compare(api, oracle_mod, sd, 3, options, settings, what=f"{kwargs} {options} {settings}")
+    _compare(api, oracle_record, sd, 3, options, settings, what=f"{kwargs} {options} {settings}")
 
 
 def test_running_mean_and_first_iteration_offset(api):
@@ -125,48 +135,48 @@ def test_running_mean_and_first_iteration_offset(api):
 
 @pytest.mark.parametrize("spectral", [False, True])
 @pytest.mark.parametrize("kind", sorted(scenes.MATERIAL_KINDS))
-def test_every_material_class_is_bit_exact(api, oracle_mod, kind, spectral):
+def test_every_material_class_is_bit_exact(api, oracle_record, kind, spectral):
     """bsdf::sample / evaluate / albedo of every Material::Class through handle_hit_ray and evaluate_light (path_tracing_shared.hxx:300-460);
     the subsurface kinds go through subsurface::gather and the per-exit emitter samples (:408-414)."""
-    _compare(api, oracle_mod, scenes.material_box(kind, 32, 32, spectral=spectral), 2, what=kind)
+    _compare(api, oracle_record, scenes.material_box(kind, 32, 32, spectral=spectral), 2, what=kind)
 
 
 @pytest.mark.parametrize("spectral", [False, True])
 @pytest.mark.parametrize("variant", [dict(), dict(sun=False, area_light=False), dict(env=False, area_light=False, textures=False)])
-def test_distant_emitters_and_textures_are_bit_exact(api, oracle_mod, variant, spectral):
+def test_distant_emitters_and_textures_are_bit_exact(api, oracle_record, variant, spectral):
     """handle_missed_ray (:462-481) over environment / directional emitters, alpha-tested and textured surfaces."""
-    _compare(api, oracle_mod, scenes.sky_room(40, 32, spectral=spectral, **variant), 2, what=str(variant))
+    _compare(api, oracle_record, scenes.sky_room(40, 32, spectral=spectral, **variant), 2, what=str(variant))
 
 
 @pytest.mark.parametrize("spectral", [False, True])
 @pytest.mark.parametrize("kind", ["fog", "cloud", "tinted", "camera"])
-def test_participating_media_are_bit_exact(api, oracle_mod, kind, spectral):
+def test_participating_media_are_bit_exact(api, oracle_record, kind, spectral):
     """try_sampling_medium / handle_sampled_medium (:259-298), Boundary crossings (:363-369), transmittance through sorted crossings."""
-    _compare(api, oracle_mod, scenes.media_box(kind, 32, 32, spectral=spectral), 2, what=kind)
+    _compare(api, oracle_record, scenes.media_box(kind, 32, 32, spectral=spectral), 2, what=kind)
 
 
 @pytest.mark.parametrize("kind", scenes.CAMERA_KINDS)
-def test_camera_variants_are_bit_exact(api, oracle_mod, kind):
-    _compare(api, oracle_mod, scenes.camera_box(kind, 32, 32, spectral=True), 2, what=kind)
+def test_camera_variants_are_bit_exact(api, oracle_record, kind):
+    _compare(api, oracle_record, scenes.camera_box(kind, 32, 32, spectral=True), 2, what=kind)
 
 
-def test_million_triangle_room_is_bit_exact(api, oracle_mod):
+def test_million_triangle_room_is_bit_exact(api, oracle_record):
     sd = scenes.procedural_room(64, 36, env_size=(256, 128))
-    _compare(api, oracle_mod, sd, 1, what="C3 room")
+    _compare(api, oracle_record, sd, 1, what="C3 room")
 
 
-def test_config4_and_config5_scenes_are_bit_exact(api, oracle_mod):
-    _compare(api, oracle_mod, scenes.sss_dragon(32, 32), 1, what="C4 subsurface mesh")
-    _compare(api, oracle_mod, scenes.cloud_box(32, 32, grid=64), 2, what="C5 cloud")
+def test_config4_and_config5_scenes_are_bit_exact(api, oracle_record):
+    _compare(api, oracle_record, scenes.sss_dragon(32, 32), 1, what="C4 subsurface mesh")
+    _compare(api, oracle_record, scenes.cloud_box(32, 32, grid=64), 2, what="C5 cloud")
 
 
-def test_reference_loaded_cornell_asset_is_bit_exact(api, oracle_mod):
+def test_reference_loaded_cornell_asset_is_bit_exact(api, oracle_record):
     """The reference loader's own PODs (committed dump): the Blackman-Harris pixel-filter image is sampled from iteration 1 on (Film::sample,
     film.cxx:137-145), fog behind a Boundary mesh, sun + sky."""
     from etx_tracer_b200 import pod_io
     sd = pod_io.load(os.path.join(GOLDEN, "ref_cornell_40.npz"))
     assert int(sd.scene["pixel_sampler_image"][0]) != S.INVALID
-    _compare(api, oracle_mod, sd, 3, what="reference Cornell asset")
+    _compare(api, oracle_record, sd, 3, what="reference Cornell asset")
 
 
 def test_adaptive_sampling_is_bit_exact(api, oracle_mod):
@@ -181,7 +191,7 @@ def test_adaptive_sampling_is_bit_exact(api, oracle_mod):
     counts = info_o & S.PIXEL_COUNT_MASK
     assert 0 < conv.sum() < conv.size, "the case must have converged and active pixels"
     assert counts.min() < n and counts.max() == n
-    _assert_bit_exact(g, o, "adaptive")
+    _assert_bit_exact(_outputs(g, sd), _outputs(o, sd), "adaptive")
     assert bit_equal(g.buffer(S.BUF_PIXEL_ERROR, np.float32), o.buffer(S.BUF_PIXEL_ERROR, np.float32))
     gs, os_ = g.pt_status(), o.pt_status()
     assert gs["active_pixels"] == os_["active_pixels"]

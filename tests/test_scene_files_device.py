@@ -35,33 +35,44 @@ def test_native_renderer_renders_what_the_python_front_end_renders(tmp_path):
     assert np.abs(pa - pb).max() <= 1
 
 
-def test_default_atmosphere_scene_renders_bit_exact_on_the_device(oracle_mod, tmp_path):
+def test_default_atmosphere_scene_renders_bit_exact_on_the_device(oracle_record, tmp_path):
     """A scene file without distant emitters: the loader adds the default sun (Directional emitter with its 128 x 128 extinction image) and sky
     (Environment emitter, 256 x 128 image with an importance table, clamped in u).  The parity build against the oracle on those PODs, both integrators."""
-    from conftest import bit_equal
+    from conftest import same_bits
     from etx_tracer_b200 import api, structs as S
     sd = api.SceneFile(_tiny_scene(tmp_path), flavor="parity")
     assert int(sd.scene["environment_emitter_count"][0]) == 2
-    o = oracle_mod.Oracle(sd)
-    o.begin(0)
-    o.run(2, threads=1)
+    buffers = ((S.BUF_LIGHT_SAMPLER, np.uint32), (S.BUF_LV_POS, np.float32), (S.BUF_CAMERA_SAMPLER, np.uint32), (S.BUF_CAMERA_GATHERED, np.float32))
+    layers = (S.FILM_CAMERA, S.FILM_NORMALS, S.FILM_ALBEDO)
+
+    def run(m):
+        o = m.Oracle(sd)
+        o.begin(0)
+        o.run(2, threads=1)
+        out = {f"vcm buffer {bid}": o.buffer(bid, dt) for bid, dt in buffers}
+        out["vcm film camera"] = o.film(S.FILM_CAMERA)[..., :3]
+        o.set_integrator(S.INTEGRATOR_PT)
+        o.pt_set_options(S.default_pt_options())
+        o.begin(0)
+        o.run(3, threads=1)
+        out["pt camera sampler"] = o.buffer(S.BUF_CAMERA_SAMPLER, np.uint32)
+        out.update({f"pt film {layer}": o.film(layer)[..., :3] for layer in layers})
+        o.close()
+        return out
+
+    ref = oracle_record("", run)
     g = api.GPUVCM(sd, flavor="parity")
     g.render(2)
-    for bid, dt in ((S.BUF_LIGHT_SAMPLER, np.uint32), (S.BUF_LV_POS, np.float32), (S.BUF_CAMERA_SAMPLER, np.uint32), (S.BUF_CAMERA_GATHERED, np.float32)):
-        assert bit_equal(g.buffer(bid, dt), o.buffer(bid, dt)), f"buffer {bid}"
-    assert bit_equal(g.film(S.FILM_CAMERA)[..., :3], o.film(S.FILM_CAMERA)[..., :3])
+    for bid, dt in buffers:
+        assert same_bits(g.buffer(bid, dt), ref[f"vcm buffer {bid}"]), f"buffer {bid}"
+    assert same_bits(g.film(S.FILM_CAMERA)[..., :3], ref["vcm film camera"])
     g.close()
-    o.set_integrator(S.INTEGRATOR_PT)
-    o.pt_set_options(S.default_pt_options())
-    o.begin(0)
-    o.run(3, threads=1)
     p = api.GPUPathTracing(sd, flavor="parity")
     p.render(3)
-    assert bit_equal(p.buffer(S.BUF_CAMERA_SAMPLER, np.uint32), o.buffer(S.BUF_CAMERA_SAMPLER, np.uint32))
-    for layer in (S.FILM_CAMERA, S.FILM_NORMALS, S.FILM_ALBEDO):
-        assert bit_equal(p.film(layer)[..., :3], o.film(layer)[..., :3]), layer
+    assert same_bits(p.buffer(S.BUF_CAMERA_SAMPLER, np.uint32), ref["pt camera sampler"])
+    for layer in layers:
+        assert same_bits(p.film(layer)[..., :3], ref[f"pt film {layer}"]), layer
     p.close()
-    o.close()
 
 
 def test_nanovdb_medium_scene_renders_bit_exact_on_the_device(oracle_mod, tmp_path):
