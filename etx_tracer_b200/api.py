@@ -25,7 +25,7 @@ class EtxbError(RuntimeError):
 def load_library(flavor="fast"):
     if flavor in _libs:
         return _libs[flavor]
-    path = os.environ.get("ETXB_LIB_" + flavor.upper()) or _build.lib_path(flavor)  # the override is for A/B experiments only
+    path = _build.lib_path(flavor)
     if not os.path.exists(path):
         raise EtxbError(-100, f"{path} is missing: run `python -c 'import __graft_entry__ as g; g.build()'` (no CPU fallback exists)")
     lib = C.CDLL(path)
@@ -39,71 +39,66 @@ def load_library(flavor="fast"):
     lib.etxb_upload_scene.argtypes = [vp, vp, u64, vp, u64]
     lib.etxb_upload_blue_noise.argtypes = [vp, vp, vp, vp]
     lib.etxb_upload_color_tables.argtypes = [vp, vp, vp]
-    if hasattr(lib, "etxb_scene_file_load"):
-        lib.etxb_scene_file_load.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(vp), C.c_char_p, u64]
-        lib.etxb_scene_file_free.argtypes = [vp]
-        lib.etxb_scene_file_free.restype = None
-        lib.etxb_scene_file_set_samples.argtypes = [vp, u32]
-        lib.etxb_scene_file_set_samples.restype = None
-        lib.etxb_scene_file_commit.argtypes = [vp, vp]
-        lib.etxb_scene_file_table.argtypes = [vp, C.c_char_p, C.POINTER(u64)]
-        lib.etxb_scene_file_table.restype = vp
-        lib.etxb_atmosphere_images.argtypes = [C.c_char_p, vp, C.c_float, vp, u32, u32, vp, vp]
-        lib.etxb_options_file_string.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, u64]
-        lib.etxb_mesh_tangents.argtypes = [vp, u64, vp, u64]
-        lib.etxb_image_file_read.argtypes = [C.c_char_p, vp, vp, vp, vp, u64, C.c_char_p, u64]
-        lib.etxb_nvdb_density.argtypes = [C.c_char_p, vp, vp, u64, C.c_char_p, u64]
-        for fn in (lib.etxb_scene_file_scene, lib.etxb_scene_file_camera):
-            fn.argtypes = [vp]
-            fn.restype = vp
-        for fn in (lib.etxb_scene_file_warning_count, lib.etxb_scene_file_material_count):
-            fn.argtypes = [vp]
-            fn.restype = u32
-        for fn in (lib.etxb_scene_file_warning, lib.etxb_scene_file_material_name):
-            fn.argtypes = [vp, u32]
-            fn.restype = C.c_char_p
+    lib.etxb_scene_file_load.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(vp), C.c_char_p, u64]
+    lib.etxb_scene_file_free.argtypes = [vp]
+    lib.etxb_scene_file_free.restype = None
+    lib.etxb_scene_file_set_samples.argtypes = [vp, u32]
+    lib.etxb_scene_file_set_samples.restype = None
+    lib.etxb_scene_file_commit.argtypes = [vp, vp]
+    lib.etxb_scene_file_table.argtypes = [vp, C.c_char_p, C.POINTER(u64)]
+    lib.etxb_scene_file_table.restype = vp
+    lib.etxb_atmosphere_images.argtypes = [C.c_char_p, vp, C.c_float, vp, u32, u32, vp, vp]
+    lib.etxb_options_file_string.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, u64]
+    lib.etxb_mesh_tangents.argtypes = [vp, u64, vp, u64]
+    lib.etxb_image_file_read.argtypes = [C.c_char_p, vp, vp, vp, vp, u64, C.c_char_p, u64]
+    lib.etxb_nvdb_density.argtypes = [C.c_char_p, vp, vp, u64, C.c_char_p, u64]
+    for fn in (lib.etxb_scene_file_scene, lib.etxb_scene_file_camera):
+        fn.argtypes = [vp]
+        fn.restype = vp
+    for fn in (lib.etxb_scene_file_warning_count, lib.etxb_scene_file_material_count):
+        fn.argtypes = [vp]
+        fn.restype = u32
+    for fn in (lib.etxb_scene_file_warning, lib.etxb_scene_file_material_name):
+        fn.argtypes = [vp, u32]
+        fn.restype = C.c_char_p
     lib.etxb_options_default.argtypes = [vp]
     lib.etxb_options_default.restype = None
     lib.etxb_options_set_key.argtypes = [vp, C.c_char_p, C.c_double]
     lib.etxb_set_options.argtypes = [vp, vp]
-    if hasattr(lib, "etxb_group_create"):
-        lib.etxb_set_next_iteration.argtypes = [vp, u32]
-        lib.etxb_group_create.argtypes = [C.POINTER(vp), vp, u32]
-        lib.etxb_group_destroy.argtypes = [vp]
-        lib.etxb_group_destroy.restype = None
-        lib.etxb_group_lanes.argtypes = [vp]
-        lib.etxb_group_lanes.restype = u32
-        lib.etxb_group_lane.argtypes = [vp, u32]
-        lib.etxb_group_lane.restype = vp
-        lib.etxb_group_last_error.argtypes = [vp]
-        lib.etxb_group_last_error.restype = C.c_char_p
-        lib.etxb_group_begin.argtypes = [vp, u32]
-        lib.etxb_group_enqueue.argtypes = [vp, u32]
-        lib.etxb_group_wait.argtypes = [vp]
-        lib.etxb_group_poll.argtypes = [vp, vp]
-        lib.etxb_group_read_film.argtypes = [vp, u32, vp, u64]
-        lib.etxb_group_set_stride.argtypes = [vp, u32]
-        lib.etxb_group_combine.argtypes = [vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u32)]
-    if hasattr(lib, "etxb_comm_init"):
-        lib.etxb_comm_unique_id.argtypes = [vp, u64]
-        lib.etxb_comm_init.argtypes = [vp, u32, u32, vp, u64]
-        lib.etxb_comm_world.argtypes = [vp, C.POINTER(u32), C.POINTER(u32)]
-        lib.etxb_comm_reduce_film.argtypes = [vp, u32, vp, u64]
-        lib.etxb_group_comm_init.argtypes = [vp, u32, u32, vp, u32]
-        lib.etxb_group_comm_reduce_film.argtypes = [vp, u32, vp, u64]
-        lib.etxb_group_comm_init_replicas.argtypes = [vp, u32, u32, vp, u64]
-        lib.etxb_group_reserve_split_lane.argtypes = [vp]
-    if hasattr(lib, "etxb_set_integrator"):
-        lib.etxb_set_integrator.argtypes = [vp, u32]
-        lib.etxb_pt_options_default.argtypes = [vp]
-        lib.etxb_pt_options_default.restype = None
-        lib.etxb_pt_options_set_key.argtypes = [vp, C.c_char_p, C.c_double]
-        lib.etxb_pt_set_options.argtypes = [vp, vp]
-        lib.etxb_pt_get_status.argtypes = [vp, vp]
-        lib.etxb_set_scene_settings.argtypes = [vp, C.c_float, C.c_float]
+    lib.etxb_set_next_iteration.argtypes = [vp, u32]
+    lib.etxb_group_create.argtypes = [C.POINTER(vp), vp, u32]
+    lib.etxb_group_destroy.argtypes = [vp]
+    lib.etxb_group_destroy.restype = None
+    lib.etxb_group_lanes.argtypes = [vp]
+    lib.etxb_group_lanes.restype = u32
+    lib.etxb_group_lane.argtypes = [vp, u32]
+    lib.etxb_group_lane.restype = vp
+    lib.etxb_group_last_error.argtypes = [vp]
+    lib.etxb_group_last_error.restype = C.c_char_p
+    lib.etxb_group_begin.argtypes = [vp, u32]
+    lib.etxb_group_enqueue.argtypes = [vp, u32]
+    lib.etxb_group_wait.argtypes = [vp]
+    lib.etxb_group_poll.argtypes = [vp, vp]
+    lib.etxb_group_read_film.argtypes = [vp, u32, vp, u64]
+    lib.etxb_group_set_stride.argtypes = [vp, u32]
+    lib.etxb_group_combine.argtypes = [vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u32)]
+    lib.etxb_comm_unique_id.argtypes = [vp, u64]
+    lib.etxb_comm_init.argtypes = [vp, u32, u32, vp, u64]
+    lib.etxb_comm_world.argtypes = [vp, C.POINTER(u32), C.POINTER(u32)]
+    lib.etxb_comm_reduce_film.argtypes = [vp, u32, vp, u64]
+    lib.etxb_group_comm_init.argtypes = [vp, u32, u32, vp, u32]
+    lib.etxb_group_comm_reduce_film.argtypes = [vp, u32, vp, u64]
+    lib.etxb_group_comm_init_replicas.argtypes = [vp, u32, u32, vp, u64]
+    lib.etxb_group_reserve_split_lane.argtypes = [vp]
+    lib.etxb_set_integrator.argtypes = [vp, u32]
+    lib.etxb_pt_options_default.argtypes = [vp]
+    lib.etxb_pt_options_default.restype = None
+    lib.etxb_pt_options_set_key.argtypes = [vp, C.c_char_p, C.c_double]
+    lib.etxb_pt_set_options.argtypes = [vp, vp]
+    lib.etxb_pt_get_status.argtypes = [vp, vp]
+    lib.etxb_set_scene_settings.argtypes = [vp, C.c_float, C.c_float]
     lib.etxb_set_partition.argtypes = [vp, u32, u32]
-    if hasattr(lib, "etxb_set_iteration_stride"):  # absent only from older builds loaded through the ETXB_LIB_* override
-        lib.etxb_set_iteration_stride.argtypes = [vp, u32]
+    lib.etxb_set_iteration_stride.argtypes = [vp, u32]
     lib.etxb_begin.argtypes = [vp, u32]
     lib.etxb_enqueue_iteration.argtypes = [vp]
     lib.etxb_enqueue_light_pass.argtypes = [vp]
@@ -114,12 +109,11 @@ def load_library(flavor="fast"):
     lib.etxb_stop.argtypes = [vp, C.c_int]
     lib.etxb_read_film.argtypes = [vp, u32, vp, u64]
     lib.etxb_film_size.argtypes = [vp, C.POINTER(u32), C.POINTER(u32)]
-    if hasattr(lib, "etxb_save_film"):
-        lib.etxb_read_film_ldr.argtypes = [vp, u32, C.c_float, vp, u64]
-        lib.etxb_save_film.argtypes = [vp, u32, C.c_char_p, u32, C.c_float]
-        lib.etxb_write_exr.argtypes = [C.c_char_p, vp, u32, u32]
-        lib.etxb_write_png.argtypes = [C.c_char_p, vp, u32, u32]
-        lib.etxb_tonemap_rgba8.argtypes = [vp, u64, C.c_float, vp]
+    lib.etxb_read_film_ldr.argtypes = [vp, u32, C.c_float, vp, u64]
+    lib.etxb_save_film.argtypes = [vp, u32, C.c_char_p, u32, C.c_float]
+    lib.etxb_write_exr.argtypes = [C.c_char_p, vp, u32, u32]
+    lib.etxb_write_png.argtypes = [C.c_char_p, vp, u32, u32]
+    lib.etxb_tonemap_rgba8.argtypes = [vp, u64, C.c_float, vp]
     lib.etxb_get_counters.argtypes = [vp, vp]
     lib.etxb_get_kernel_times.argtypes = [vp, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.POINTER(u32), u32]
     lib.etxb_read_buffer.argtypes = [vp, u32, vp, u64, C.POINTER(u64)]
@@ -127,8 +121,7 @@ def load_library(flavor="fast"):
     lib.etxb_stream.restype = vp
     lib.etxb_stream.argtypes = [vp]
     lib.etxb_debug_trace.argtypes = [vp, vp, vp, u32, vp, vp]
-    if hasattr(lib, "etxb_debug_select_tree"):
-        lib.etxb_debug_select_tree.argtypes = [vp, C.c_int]
+    lib.etxb_debug_select_tree.argtypes = [vp, C.c_int]
     lib.etxb_debug_sampler.argtypes = [vp, vp, vp, u32, u32, vp, vp]
     lib.etxb_debug_math.argtypes = [vp, u32, vp, vp, u32, vp]
     _libs[flavor] = lib

@@ -3,6 +3,9 @@
   libetx_b200.so         product build ("fast": FMA contraction, CUDA math library)
   libetx_b200_parity.so  strict-IEEE build (-fmad=false, portable transcendentals) used by the bit-exact parity tests
   libetx_b200_count.so   product build + traversal counters (bench.py roofline pass)
+
+The alternatives measured against "fast" (round 1's IEEE division / sqrt with the CUDA math library; other resident-block counts for the
+bounce, connection and gather kernels) are recorded in DESIGN.md §5 and the constants in kernels.cuh; they are not built.
 """
 import os
 import subprocess
@@ -22,13 +25,6 @@ FLAVORS = {
     # "fast" + per-ray node / triangle counters in every traversal (bench.py's roofline pass reads n_node / n_tri from it: SURVEY 8(d) wants the
     # algorithmic bytes with and without the BVH term; the counters cost registers, so the timed build does not carry them)
     "count": (os.path.join(HERE, "libetx_b200_count.so"), ["-prec-div=false", "-prec-sqrt=false", "-ftz=true", "-DETXB_COUNT_TRAVERSAL=1"]),
-    # A/B partners of "fast": the bounce / connection kernels compiled for 3 or 2 resident blocks per SM (168 / 255 registers: fewer spills, fewer warps)
-    "fast_mb3": (os.path.join(HERE, "libetx_b200_mb3.so"), ["-prec-div=false", "-prec-sqrt=false", "-ftz=true", "-DETXB_BOUNCE_MIN_BLOCKS=3", "-DETXB_CONNECT_MIN_BLOCKS=3"]),
-    "fast_mb2": (os.path.join(HERE, "libetx_b200_mb2.so"), ["-prec-div=false", "-prec-sqrt=false", "-ftz=true", "-DETXB_BOUNCE_MIN_BLOCKS=2", "-DETXB_CONNECT_MIN_BLOCKS=2"]),
-    # A/B partner of "fast": the closure gather compiled for 3 resident blocks per SM (168 registers, no spills) instead of 4 (128)
-    "fast_cl3": (os.path.join(HERE, "libetx_b200_cl3.so"), ["-prec-div=false", "-prec-sqrt=false", "-ftz=true", "-DETXB_CLOSURE_MIN_BLOCKS=3"]),
-    # A/B partner of "fast": round 1's arithmetic (IEEE division / sqrt, CUDA math library)
-    "fast_precise": (os.path.join(HERE, "libetx_b200_precise.so"), ["-DETXB_PRECISE_MATH=1"]),
     "parity": (os.path.join(HERE, "libetx_b200_parity.so"), ["-fmad=false", "-DETXB_PARITY=1"]),
 }
 

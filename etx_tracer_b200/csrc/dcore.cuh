@@ -58,21 +58,6 @@ DEVN float m_cosh(float x) { return pm::coshf_(x); }
 DEVN float m_atanh(float x) { return pm::atanhf_(x); }
 DEVN float m_sinh(float x) { return pm::sinhf_(x); }
 DEVN float m_tanh(float x) { return pm::tanhf_(x); }
-#elif defined(ETXB_PRECISE_MATH)
-// A/B switch: the CUDA math library's full-precision routines (what round 1 shipped)
-DEV float m_sin(float x) { return sinf(x); }
-DEV float m_cos(float x) { return cosf(x); }
-DEV float m_exp(float x) { return expf(x); }
-DEV float m_log(float x) { return logf(x); }
-DEVG_MATH float m_pow(float x, float y) { return powf(x, y); }
-DEVG_MATH float m_acos(float x) { return acosf(x); }
-DEVG_MATH float m_asin(float x) { return asinf(x); }
-DEVG_MATH float m_atan(float x) { return atanf(x); }
-DEVG_MATH float m_atan2(float y, float x) { return atan2f(y, x); }
-DEVG_MATH float m_cosh(float x) { return coshf(x); }
-DEVG_MATH float m_atanh(float x) { return atanhf(x); }
-DEVG_MATH float m_sinh(float x) { return sinhf(x); }
-DEVG_MATH float m_tanh(float x) { return tanhf(x); }
 #else
 // Product build: the special-function unit.  sin / cos / exp2 / log2 are single MUFU instructions (2^-21 absolute error on the reduced
 // range); the library routines they replace are 40-150 instructions each and were inlined at ~100 sites of the BSDF code, which made the

@@ -902,7 +902,7 @@ DEV Spec<SP> vcm_connection_transmittance(const DeviceScene& sc, const Endpoint&
 // vcm_connect_to_light_path (vcm_shared.hxx:765-803): serial over the paired path's vertices (shared sampler)
 template <bool SP, bool PLAIN = false>
 DEV Spec<SP> vcm_connect_to_light_path(const DeviceScene& sc, const VcmParams& it, const LightVertexRec* pool, uint32_t lp_index, uint32_t lp_count, const Endpoint& ep,
-  PathState<SP>& state, TraverseStats* stats, uint32_t& shadow_rays, uint32_t& connections, ShadowBatch* batch = nullptr) {
+  PathState<SP>& state, TraverseStats* stats, uint32_t& shadow_rays, uint32_t& connections) {
   Spec<SP> result = Spec<SP>::make(0.0f);
   if (it.connect_vertices() == false) return result;
   for (uint32_t i = 0; i < lp_count; ++i) {
@@ -915,12 +915,6 @@ DEV Spec<SP> vcm_connect_to_light_path(const DeviceScene& sc, const VcmParams& i
     Spec<SP> value;
     if (vcm_connect_to_light_vertex<SP>(sc, it, state, lv, ep, target_position, value)) {
       shadow_rays += 1;
-      if (batch != nullptr) {  // surface endpoints only
-        const Isect& isect = *ep.isect;
-        V3 p0 = shading_pos(sc, load_triangle(sc, isect.triangle_index), isect.barycentric, normalize(target_position - isect.pos));
-        batch->push<SP>(p0, target_position, value);
-        continue;
-      }
       Spec<SP> tr = vcm_connection_transmittance<SP, PLAIN>(sc, ep, lv, target_position, state, stats);
       if (tr.is_zero() == false) {
         result += tr * value;

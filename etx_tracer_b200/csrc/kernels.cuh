@@ -19,14 +19,10 @@
 
 // resident blocks per SM the bounce / connection kernels are compiled for (128 threads each: 4 blocks = 128 registers per thread).
 // Measured on the B200 (bench.py --lanes 1): 1|1 -> 4|4 gives C2 11.04 -> 11.36 and C3 5.55 -> 5.79 Msamples/s; 2 and 3 change nothing.
-#ifndef ETXB_BOUNCE_MIN_BLOCKS
-#define ETXB_BOUNCE_MIN_BLOCKS 4
-#endif
-#ifndef ETXB_CONNECT_MIN_BLOCKS
-#define ETXB_CONNECT_MIN_BLOCKS 4
-#endif
-
 namespace etxb {
+
+constexpr int kBounceMinBlocks = 4;
+constexpr int kConnectMinBlocks = 4;
 
 struct PathBuffers {
   float4* ray_o;     // o.xyz, min_t
@@ -96,12 +92,7 @@ struct LaunchParams {
   uint32_t shadow_stage;         // 1: the scene qualifies (DeviceScene::deferred_shadow_rays) and the buffers exist
   uint32_t shadow_atomic;        // 1 (product build, opaque scenes with stochastic BSDFs): the shadow segments of NEE, vertex connections and
                                  //    light-to-camera connections go to the shadow list with their target address; k_shadow_resolve adds the unoccluded ones
-  uint32_t closures;             // 1 (product build): connections and the generic gather evaluate vertex closures (dclosure.cuh); 0: A/B switch
-  uint32_t merge_material_major; // 1: the gather queue is ordered by (material, Morton code) instead of the Morton code alone (ETXB_MERGE_MATERIAL_MAJOR=1)
-  uint32_t spatial_keys;         // 1 (experiment, ETXB_QUEUE_SORT_SPATIAL=1): the path-queue sort key is (hit material, Morton code of the hit point) instead of the
-                                 //    material alone — the next bounce's rays then start from neighbouring points in neighbouring queue slots
-  uint32_t connect_deferred;     // 1 (needs shadow_stage): the camera-vertex x light-vertex connections of such a scene run one per thread in
-                                 //    k_camera_connect_deferred — conn_list[slot] names the (path, light vertex) pair that fills shadow slot `slot`
+  uint32_t merge_material_major; // 1 (scenes with stochastic BSDFs): the gather queue is ordered by (material, Morton code) instead of the Morton code alone
 };
 
 #ifdef ETXB_COUNT_TRAVERSAL
@@ -209,28 +200,9 @@ __global__ void __launch_bounds__(128) k_light_begin(const __grid_constant__ Lau
   queue_push(queue, queue_count, alive, i);
 }
 
-// Sort key of a queue slot after its closest-hit query: the hit material (0xff = miss; 0x100 = slot past the device-side count, sorts last); with
-// p.spatial_keys the material moves to bits 23-31 and bits 0-22 hold the top of the 30-bit Morton code of the hit point inside the scene's bounding cube
+// Sort key of a queue slot after its closest-hit query: the hit material (0xff = miss; 0x100 = slot past the device-side count, sorts last)
 constexpr uint32_t kQueueKeyPastCount = 0x100u;
-DEV uint32_t spread10(uint32_t v) {
-  v = (v | (v << 16)) & 0x030000FFu;
-  v = (v | (v << 8)) & 0x0300F00Fu;
-  v = (v | (v << 4)) & 0x030C30C3u;
-  v = (v | (v << 2)) & 0x09249249u;
-  return v;
-}
-DEV uint32_t queue_sort_key(const LaunchParams& p, uint32_t tri, float4 o, float4 d, float t) {
-  const uint32_t material = (tri == kInvalidIndex) ? 0xffu : umin(load_triangle_material(p.scene, tri), 0xfeu);
-  if (!p.spatial_keys) return material;
-  const float r = p.scene.bounding_sphere_radius, s = 1024.0f / fmaxf(2.0f * r, 1e-20f);
-  const float tt = (tri == kInvalidIndex) ? 0.0f : t;
-  const V3 c = p.scene.bounding_sphere_center;
-  uint32_t x = umin(uint32_t(fmaxf((o.x + d.x * tt - (c.x - r)) * s, 0.0f)), 1023u);
-  uint32_t y = umin(uint32_t(fmaxf((o.y + d.y * tt - (c.y - r)) * s, 0.0f)), 1023u);
-  uint32_t z = umin(uint32_t(fmaxf((o.z + d.z * tt - (c.z - r)) * s, 0.0f)), 1023u);
-  return (material << 23) | ((spread10(x) | (spread10(y) << 1) | (spread10(z) << 2)) >> 7);
-}
-DEV uint32_t queue_key_past_count(const LaunchParams& p) { return p.spatial_keys ? (kQueueKeyPastCount << 23) : kQueueKeyPastCount; }
+DEV uint32_t queue_sort_key(const LaunchParams& p, uint32_t tri) { return (tri == kInvalidIndex) ? 0xffu : umin(load_triangle_material(p.scene, tri), 0xfeu); }
 
 // closest-hit traversal for every queued path (Raytracing::trace, rt.cxx:428): SoA ray in, hit record out,
 // sampler advanced by one draw per candidate
@@ -238,7 +210,7 @@ __global__ void __launch_bounds__(256) k_trace_closest(const __grid_constant__ L
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= *queue_count) {
     // the host sorts `key_limit` (its upper bound of the queue size) slots by material: slots past the device-side count sort last
-    if ((material_keys != nullptr) && (q < key_limit)) material_keys[q] = queue_key_past_count(p);
+    if ((material_keys != nullptr) && (q < key_limit)) material_keys[q] = kQueueKeyPastCount;
     return;
   }
   uint32_t i = queue[q];
@@ -252,7 +224,7 @@ __global__ void __launch_bounds__(256) k_trace_closest(const __grid_constant__ L
   p.paths.hit[i] = make_float4(h.u, h.v, h.t, __uint_as_float(h.tri));
   p.paths.misc[i].x = smp.seed;
   // the bounce kernels' cost is the BSDF class of the surface that was hit: paths are grouped by material before they are shaded
-  if (material_keys != nullptr) material_keys[q] = queue_sort_key(p, h.tri, o, d, h.t);
+  if (material_keys != nullptr) material_keys[q] = queue_sort_key(p, h.tri);
   counter_add(&p.counters->rays_closest, 1u);
   counter_add(&p.counters->nodes, STATS_NODES);
   counter_add(&p.counters->tris, STATS_TRIS);
@@ -315,7 +287,7 @@ enum : uint32_t { kEpNone = 0u, kEpMedium = 1u, kEpSurface = 2u, kEpSubsurface =
 // the segment (medium scattering, boundary crossing, surface hit incl. the subsurface walk), (B) camera connections from the
 // endpoint(s) it produced — one, or every gathered subsurface exit (:1207-1222), (C) the continuation.
 template <bool SP, bool PLAIN>
-__global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_light_bounce(const __grid_constant__ LaunchParams p, const uint32_t* queue_in, const uint32_t* count_in, uint32_t* queue_out, uint32_t* count_out) {
+__global__ void __launch_bounds__(128, kBounceMinBlocks) k_light_bounce(const __grid_constant__ LaunchParams p, const uint32_t* queue_in, const uint32_t* count_in, uint32_t* queue_out, uint32_t* count_out) {
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   bool alive = false;
   uint32_t i = 0;
@@ -673,7 +645,7 @@ DEV void camera_emit_connections(const LaunchParams& p, uint32_t i, uint32_t cam
 // the paired light path and to a sampled emitter from the endpoint(s) the event produced (one, or every gathered subsurface exit,
 // :1037-1053), (C) the MIS update / pending continuation sample handed to the merge and continue stages.
 template <bool SP, bool PLAIN>
-__global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_camera_shade(const __grid_constant__ LaunchParams p, const uint32_t* queue_in, const uint32_t* count_in) {
+__global__ void __launch_bounds__(128, kBounceMinBlocks) k_camera_shade(const __grid_constant__ LaunchParams p, const uint32_t* queue_in, const uint32_t* count_in) {
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t shadow_rays = 0, connections = 0;
   uint32_t merge_key = 0xffffffffu;
@@ -790,7 +762,7 @@ __global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_camera_shade(co
           } else if (p.connect_stage && (ep_mode == kEpSurface)) {
             camera_emit_connections<SP>(p, i, isect.material_index, state, connections);
             continue;
-          } else if (deferred && p.connect_deferred) {
+          } else if (deferred) {
             // one slot per connection of this vertex, in the reference's order (vcm_shared.hxx:765-803); k_camera_connect_deferred
             // evaluates each pair in its own thread and fills (or voids) the slot — no BSDF of such a scene draws from the sampler
             if (p.vcm.connect_vertices()) {
@@ -805,8 +777,7 @@ __global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_camera_shade(co
             continue;
           } else {
             // reference order: serial over the paired path's vertices with the path's own sampler
-            c = vcm_connect_to_light_path<SP, PLAIN>(sc, p.vcm, p.lv_final, p.lp_offset[i], p.paths.lv_count[i], ep, state, stats, shadow_rays, connections, deferred);
-            if (deferred) shadow_span.y = batch.count;  // segments to light vertices come first, the emitter segment (if any) last
+            c = vcm_connect_to_light_path<SP, PLAIN>(sc, p.vcm, p.lv_final, p.lp_offset[i], p.paths.lv_count[i], ep, state, stats, shadow_rays, connections);
           }
           state.gathered += (ep_mode == kEpSubsurface) ? (w * c) : c;
         }
@@ -819,9 +790,7 @@ __global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_camera_shade(co
         // reserved slots that were not used (failed connections, or a reservation that ran past the capacity) are marked empty
         for (uint32_t k = batch.base + batch.count; (k < batch.base + reserved) && (k < p.shadow_capacity); ++k) p.shadow_p0[k].w = -1.0f;
         // slots that are no vertex connection (the emitter segment, unused ones) carry no pair
-        if (p.connect_deferred) {
-          for (uint32_t k = batch.base + (shadow_span.y & 0xffffu); (k < batch.base + reserved) && (k < p.shadow_capacity); ++k) p.conn_list[k].x = kInvalidIndex;
-        }
+        for (uint32_t k = batch.base + (shadow_span.y & 0xffffu); (k < batch.base + reserved) && (k < p.shadow_capacity); ++k) p.conn_list[k].x = kInvalidIndex;
       }
     }
     if (p.shadow_stage) p.paths.shadow_span[i] = shadow_span;
@@ -860,8 +829,8 @@ __global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_camera_shade(co
       }
       if (is_connectible && p.vcm.merge_vertices() && (state.total_path_depth + 1 <= sc.max_path_length) && (p.grid.photon_count != 0u)) {
         merge_key = merge_query_key(p.grid, isect.pos);
-        // experiment switch (default off, not yet measured): material-major order of the gather queue, so that the warps in flight evaluate ONE
-        // BSDF class at a time (ncu: k_camera_merge_generic_batched waits on instruction fetch, profiles/r1b_c3_k_*.raw.csv)
+        // material-major order of the gather queue, so that the warps in flight evaluate ONE BSDF class at a time (the generic gather waited on
+        // instruction fetch, profiles/r1b_c3_k_*.raw.csv; measured on the B200, round 2: C3 generic gather 60.6 -> 46.1 ms per iteration)
         if (p.merge_material_major && (merge_key != 0xffffffffu)) merge_key = (umin(isect.material_index, 0x7eu) << 24) | (merge_key >> 6);
       }
       V3 w = bs.weight.as_v3();
@@ -943,7 +912,7 @@ DEV bool vcm_connect_to_light_vertex_closure(const DeviceScene& sc, const VcmPar
 // vcm_connect_to_light_path (vcm_shared.hxx:673-803).  Each connection draws from its own stream derived from the path's sampler
 // (the reference shares one stream across the serial loop; the parity build keeps that order inside k_camera_shade).
 template <bool SP, bool PLAIN>
-__global__ void __launch_bounds__(128, ETXB_CONNECT_MIN_BLOCKS) k_camera_connect(const __grid_constant__ LaunchParams p, const uint2* conn_list) {
+__global__ void __launch_bounds__(128, kConnectMinBlocks) k_camera_connect(const __grid_constant__ LaunchParams p, const uint2* conn_list) {
   uint32_t shadow_rays = 0;
   STATS_DECL;
   const DeviceScene& sc = p.scene;
@@ -965,8 +934,7 @@ __global__ void __launch_bounds__(128, ETXB_CONNECT_MIN_BLOCKS) k_camera_connect
 #if defined(ETXB_PARITY) && ETXB_PARITY
     const bool connected = vcm_connect_to_light_vertex<SP>(sc, p.vcm, state, lv, ep, target_position, value);
 #else
-    const bool connected = p.closures ? vcm_connect_to_light_vertex_closure<SP>(sc, p.vcm, state, lv, isect, target_position, value)
-                                      : vcm_connect_to_light_vertex<SP>(sc, p.vcm, state, lv, ep, target_position, value);
+    const bool connected = vcm_connect_to_light_vertex_closure<SP>(sc, p.vcm, state, lv, isect, target_position, value);
 #endif
     if (connected && PLAIN && p.shadow_atomic) {
       shadow_rays += 1;
@@ -997,7 +965,7 @@ __global__ void __launch_bounds__(128, ETXB_CONNECT_MIN_BLOCKS) k_camera_connect
 // connection that succeeds writes the slot's segment and unoccluded contribution (k_shadow_trace resolves it, k_camera_continue adds the
 // visible ones in slot order = reference order); one that fails voids the slot.  Same values, same order as the serial loop.
 template <bool SP>
-__global__ void __launch_bounds__(128, ETXB_CONNECT_MIN_BLOCKS) k_camera_connect_deferred(const __grid_constant__ LaunchParams p) {
+__global__ void __launch_bounds__(128, kConnectMinBlocks) k_camera_connect_deferred(const __grid_constant__ LaunchParams p) {
   const uint32_t total = umin(p.shadow_count[0], p.shadow_capacity);
   const DeviceScene& sc = p.scene;
   uint32_t shadow_rays = 0;
@@ -1073,12 +1041,8 @@ __global__ void __launch_bounds__(128) k_camera_merge_serial(const __grid_consta
 constexpr uint32_t kMergeWarpsPerBlock = 8;
 constexpr uint32_t kMergeListSize = 64;
 
-// GENERIC = false: Lambert camera vertices (BSDF value independent of the photon direction, no sampler use).
-// GENERIC = true : every other class (microfacet walks, mixtures).  Their evaluate()/pdf() are stochastic; in the product build
-//                  each in-radius photon is evaluated by its own lane with a lane-local sampler derived from (path seed, photon
-//                  index), and the path's sampler advances by one draw per query — statistically equivalent to the reference's
-//                  serial order (which the parity build keeps), 32x more parallel.
-template <bool SP, bool GENERIC>
+// Lambert camera vertices only (BSDF value independent of the photon direction, no sampler use); k_camera_merge_closure gathers the others.
+template <bool SP>
 __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(const __grid_constant__ LaunchParams p, const uint32_t* sorted_ids, const uint32_t* sorted_keys, const uint32_t* count_in,
                                                                                 uint32_t queries_per_warp) {
   __shared__ uint32_t s_idx[kMergeWarpsPerBlock][kMergeListSize];
@@ -1097,18 +1061,13 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
   V3 qpos = {0, 0, 0}, qnrm = {0, 0, 0}, qfn = {0, 0, 0}, qc = {0, 0, 0};
   float q_wcam_base = 0.0f, q_dvm = 0.0f, q_rev_cos = 0.0f;
   uint32_t q_depth = 0;
-  // GENERIC only: the rest of the camera vertex
-  V3 qtan = {0, 0, 0}, qbtn = {0, 0, 0}, qwi = {0, 0, 0};
-  V2 qtex = {0, 0};
-  float q_wavelength = 0.0f;
-  uint32_t q_medium = 0, q_material = 0, q_seed = 0;
   if (coop_active) {
     i = sorted_ids[q];
     float4 hit = p.paths.hit[i];
     PathState<SP> state = load_state<SP>(p.paths, i);
     Isect isect = stage_intersection<SP>(p, state, i, hit);
     const etxb_material& mat = sc.materials[isect.material_index];
-    coop_active = merge_is_lambert(mat) != GENERIC;
+    coop_active = merge_is_lambert(mat);
     if (coop_active) {
       merge_queries = 1;
       qpos = isect.pos;
@@ -1117,25 +1076,11 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
       q_dvm = state.d_vm;
       q_depth = state.total_path_depth;
       Spec<SP> t_camera = state.throughput / sampling_pdf<SP>(state.wavelength);
-      if constexpr (!GENERIC) {
-        bool entering = dot(isect.nrm, isect.w_i) < 0.0f;
-        qfn = entering ? isect.nrm : -isect.nrm;  // frame normal of the camera vertex
-        Spec<SP> diffuse = apply_image<SP>(sc, mat.scattering, isect.tex, state.wavelength);
-        qc = spec_to_rgb<SP>(sc, (diffuse / kPi) * t_camera, state.wavelength);  // camera_bsdf.func * t_camera: direction independent
-        q_rev_cos = dot(isect.nrm, -isect.w_i);  // reverse pdf = cos between -w_i(camera) and the normal facing the photon (bsdf_various.hxx:113-121)
-      } else {
-        qc = t_camera.as_v3();
-        qtan = isect.tan;
-        qbtn = isect.btn;
-        qwi = isect.w_i;
-        qtex = isect.tex;
-        q_wavelength = state.wavelength;
-        q_medium = state.medium_index;
-        q_material = isect.material_index;
-        q_seed = state.sampler.seed;
-        state.sampler.next();  // the path's own stream moves on by one draw per query
-        p.paths.misc[i].x = state.sampler.seed;
-      }
+      bool entering = dot(isect.nrm, isect.w_i) < 0.0f;
+      qfn = entering ? isect.nrm : -isect.nrm;  // frame normal of the camera vertex
+      Spec<SP> diffuse = apply_image<SP>(sc, mat.scattering, isect.tex, state.wavelength);
+      qc = spec_to_rgb<SP>(sc, (diffuse / kPi) * t_camera, state.wavelength);  // camera_bsdf.func * t_camera: direction independent
+      q_rev_cos = dot(isect.nrm, -isect.w_i);  // reverse pdf = cos between -w_i(camera) and the normal facing the photon (bsdf_various.hxx:113-121)
     }
   }
   uint32_t pending = __ballot_sync(0xffffffffu, coop_active);
@@ -1154,21 +1099,6 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
     float b_dvm = __shfl_sync(0xffffffffu, q_dvm, src);
     float b_rev_cos = __shfl_sync(0xffffffffu, q_rev_cos, src);
     uint32_t b_depth = __shfl_sync(0xffffffffu, q_depth, src);
-    BData cam = {};
-    uint32_t b_material = 0, b_seed = 0;
-    if constexpr (GENERIC) {
-      cam.pos = bpos;
-      cam.nrm = bnrm;
-      cam.tan = {__shfl_sync(0xffffffffu, qtan.x, src), __shfl_sync(0xffffffffu, qtan.y, src), __shfl_sync(0xffffffffu, qtan.z, src)};
-      cam.btn = {__shfl_sync(0xffffffffu, qbtn.x, src), __shfl_sync(0xffffffffu, qbtn.y, src), __shfl_sync(0xffffffffu, qbtn.z, src)};
-      cam.w_i = {__shfl_sync(0xffffffffu, qwi.x, src), __shfl_sync(0xffffffffu, qwi.y, src), __shfl_sync(0xffffffffu, qwi.z, src)};
-      cam.tex = {__shfl_sync(0xffffffffu, qtex.x, src), __shfl_sync(0xffffffffu, qtex.y, src)};
-      cam.wavelength = __shfl_sync(0xffffffffu, q_wavelength, src);
-      cam.current_medium = __shfl_sync(0xffffffffu, q_medium, src);
-      cam.path_source = kPathCamera;
-      b_material = __shfl_sync(0xffffffffu, q_material, src);
-      b_seed = __shfl_sync(0xffffffffu, q_seed, src);
-    }
     // the eight cells (vcm_shared.hxx:895-916): lanes 0..7 fetch their ranges, then an 8-wide exclusive scan of the counts
     // (prefetching the next query's ranges and the next 32 candidate positions was measured: no gain, the sweep is L2-bandwidth bound)
     uint32_t my_begin = 0, my_cnt = 0;
@@ -1209,40 +1139,20 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
         float4 lt = __ldg(&g.thr_rgb[j]);
         bool ok = !(__float_as_uint(wl.w) + b_depth + 1 > sc.max_path_length);
         ok = ok && !(dot(bnrm, V3{nd.x, nd.y, nd.z}) <= kEpsilon);
-        float bsdf_pdf_v = 0.0f, rev_pdf = 0.0f;
-        V3 c_value = {1.0f, 1.0f, 1.0f};
-        if constexpr (!GENERIC) {
-          float cos_o = -(bfn.x * wl.x + bfn.y * wl.y + bfn.z * wl.z);  // local_w_o.z of DiffuseBSDF::evaluate(-w_in)
-          ok = ok && (cos_o > kEpsilon);
-          bsdf_pdf_v = kInvPi * cos_o;
-          float facing = (dot(bnrm, V3{wl.x, wl.y, wl.z}) < 0.0f) ? b_rev_cos : -b_rev_cos;
-          rev_pdf = (facing <= kEpsilon) ? 0.0f : kInvPi * facing;
-        } else {
-          if (ok) {
-            Smp lane_smp;
-            lane_smp.seed = b_seed ^ ((j + 1u) * 0x9E3779B1u);
-            lane_smp.fixed_u = lane_smp.fixed_v = lane_smp.fixed_w = 0.0f;
-            lane_smp.next();
-            const etxb_material& mat = sc.materials[b_material];
-            V3 wo = {-wl.x, -wl.y, -wl.z};
-            BEval<SP> e = bsdf_evaluate<SP>(sc, cam, wo, mat, lane_smp);
-            ok = e.valid();
-            if (ok) {
-              rev_pdf = bsdf_reverse_pdf<SP>(sc, cam, wo, mat, lane_smp);
-              bsdf_pdf_v = e.pdf;
-              c_value = spec_to_rgb<SP>(sc, e.func * Spec<SP>::make3(bqc), cam.wavelength);
-            }
-          }
-        }
+        float cos_o = -(bfn.x * wl.x + bfn.y * wl.y + bfn.z * wl.z);  // local_w_o.z of DiffuseBSDF::evaluate(-w_in)
+        ok = ok && (cos_o > kEpsilon);
+        float bsdf_pdf_v = kInvPi * cos_o;
+        float facing = (dot(bnrm, V3{wl.x, wl.y, wl.z}) < 0.0f) ? b_rev_cos : -b_rev_cos;
+        float rev_pdf = (facing <= kEpsilon) ? 0.0f : kInvPi * facing;
         if (ok) {
           float w_light = dvcm * vc_weight + nd.w * bsdf_pdf_v;
           float w_camera = b_wcam_base + b_dvm * rev_pdf;
           float weight = use_mis ? (1.0f / (1.0f + w_light + w_camera)) : 1.0f;
           float kernel_weight = use_epan ? fmaxf(2.0f * (1.0f - distance_squared * g.inv_radius_squared), 0.0f) : 1.0f;
           float kw = kernel_weight * weight;
-          wx += c_value.x * lt.x * kw;
-          wy += c_value.y * lt.y * kw;
-          wz += c_value.z * lt.z * kw;
+          wx += lt.x * kw;
+          wy += lt.y * kw;
+          wz += lt.z * kw;
           accepts += 1;
         }
       }
@@ -1306,7 +1216,7 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
     if (lane == src) {
       V3 l = {wx, wy, wz};
       if (SP) l *= V3{0.817660332f, 1.05418909f, 1.09945524f};  // kRGBLuminanceScale (:876-878)
-      my_sum = GENERIC ? l : qc * l;
+      my_sum = qc * l;
     }
   }
   if (merge_queries) {
@@ -1318,235 +1228,22 @@ __global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_coop(
   counter_add(&p.counters->merge_accepts, accepts);
 }
 
-// Generic gather with the evaluations batched ACROSS the queries of a warp.  k_camera_merge_coop<SP, true> evaluates the in-radius photons
-// of one query at a time, 32 per step: a query with 20 of them leaves 12 lanes idle through two stochastic BSDF evaluations.  Here the
-// (query, photon) pairs of all the warp's queries go through one shared list; a step takes 32 pairs whatever query they belong to, each
-// lane fetches ITS query's camera vertex from the owning lane by shuffle, and the contributions meet in per-query shared accumulators.
-// Same pairs, same per-pair streams (path seed x photon index) as the per-query kernel; only the summation order differs.
-template <bool SP>
-__global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_generic_batched(const __grid_constant__ LaunchParams p, const uint32_t* sorted_ids, const uint32_t* sorted_keys,
-                                                                                           const uint32_t* count_in, uint32_t queries_per_warp) {
-  __shared__ uint32_t s_idx[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_d2[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_dvcm[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ uint32_t s_src[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_sum[kMergeWarpsPerBlock][32][3];
-  constexpr uint32_t kFull = 0xffffffffu;
-  const DeviceScene& sc = p.scene;
-  const GridData& g = p.grid;
-  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  const uint32_t lane_lt = (1u << lane) - 1u;
-  uint32_t q = ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * queries_per_warp + lane;
-  uint32_t merge_queries = 0, candidates = 0, accepts = 0;
-  bool active = (lane < queries_per_warp) && (q < *count_in) && (sorted_keys[q] != 0xffffffffu);
-  uint32_t i = 0;
-  // this lane's query: the camera vertex and what its MIS weight needs
-  V3 qpos = {0, 0, 0}, qnrm = {0, 0, 0}, qtan = {0, 0, 0}, qbtn = {0, 0, 0}, qwi = {0, 0, 0}, qc = {0, 0, 0};
-  V2 qtex = {0, 0};
-  float q_wcam_base = 0.0f, q_dvm = 0.0f, q_wavelength = 0.0f;
-  uint32_t q_depth = 0, q_medium = 0, q_material = 0, q_seed = 0;
-  if (active) {
-    i = sorted_ids[q];
-    float4 hit = p.paths.hit[i];
-    PathState<SP> state = load_state<SP>(p.paths, i);
-    Isect isect = stage_intersection<SP>(p, state, i, hit);
-    active = !merge_is_lambert(sc.materials[isect.material_index]);
-    if (active) {
-      merge_queries = 1;
-      qpos = isect.pos;
-      qnrm = isect.nrm;
-      qtan = isect.tan;
-      qbtn = isect.btn;
-      qwi = isect.w_i;
-      qtex = isect.tex;
-      q_wcam_base = state.d_vcm * p.vcm.vc_weight;
-      q_dvm = state.d_vm;
-      q_depth = state.total_path_depth;
-      qc = (state.throughput / sampling_pdf<SP>(state.wavelength)).as_v3();
-      q_wavelength = state.wavelength;
-      q_medium = state.medium_index;
-      q_material = isect.material_index;
-      q_seed = state.sampler.seed;
-      state.sampler.next();  // the path's own stream moves on by one draw per query
-      p.paths.misc[i].x = state.sampler.seed;
-    }
-  }
-  s_sum[warp][lane][0] = 0.0f;
-  s_sum[warp][lane][1] = 0.0f;
-  s_sum[warp][lane][2] = 0.0f;
-  __syncwarp();
-  uint32_t pending = __ballot_sync(kFull, active);
-  const bool use_mis = p.vcm.enable_mis();
-  const bool use_epan = (p.vcm.kernel == 1u);
-  const float vc_weight = p.vcm.vc_weight;
-  uint32_t n_list = 0;  // warp-uniform fill of the shared pair list
-
-  auto shfl3 = [&](V3 v, uint32_t s) { return V3{__shfl_sync(kFull, v.x, s), __shfl_sync(kFull, v.y, s), __shfl_sync(kFull, v.z, s)}; };
-  auto finish = [&](uint32_t n) {
-    // lanes < n take one (query, photon) pair; every lane takes part in the shuffles that fetch its pair's query
-    uint32_t j = 0, s = 0;
-    float distance_squared = 0.0f, dvcm = 0.0f;
-    if (lane < n) {
-      j = s_idx[warp][lane];
-      distance_squared = s_d2[warp][lane];
-      dvcm = s_dvcm[warp][lane];
-      s = s_src[warp][lane];
-    }
-    BData cam = {};
-    cam.pos = shfl3(qpos, s);
-    cam.nrm = shfl3(qnrm, s);
-    cam.tan = shfl3(qtan, s);
-    cam.btn = shfl3(qbtn, s);
-    cam.w_i = shfl3(qwi, s);
-    cam.tex = {__shfl_sync(kFull, qtex.x, s), __shfl_sync(kFull, qtex.y, s)};
-    cam.wavelength = __shfl_sync(kFull, q_wavelength, s);
-    cam.current_medium = __shfl_sync(kFull, q_medium, s);
-    cam.path_source = kPathCamera;
-    V3 bqc = shfl3(qc, s);
-    float b_wcam_base = __shfl_sync(kFull, q_wcam_base, s);
-    float b_dvm = __shfl_sync(kFull, q_dvm, s);
-    uint32_t b_depth = __shfl_sync(kFull, q_depth, s);
-    uint32_t b_material = __shfl_sync(kFull, q_material, s);
-    uint32_t b_seed = __shfl_sync(kFull, q_seed, s);
-    if (lane < n) {
-      float4 wl = __ldg(&g.win_len[j]);
-      float4 nd = __ldg(&g.nrm_dvm[j]);
-      float4 lt = __ldg(&g.thr_rgb[j]);
-      bool ok = !(__float_as_uint(wl.w) + b_depth + 1 > sc.max_path_length);
-      ok = ok && !(dot(cam.nrm, V3{nd.x, nd.y, nd.z}) <= kEpsilon);
-      if (ok) {
-        Smp lane_smp;
-        lane_smp.seed = b_seed ^ ((j + 1u) * 0x9E3779B1u);
-        lane_smp.fixed_u = lane_smp.fixed_v = lane_smp.fixed_w = 0.0f;
-        lane_smp.next();
-        const etxb_material& mat = sc.materials[b_material];
-        V3 wo = {-wl.x, -wl.y, -wl.z};
-        BEval<SP> e = bsdf_evaluate<SP>(sc, cam, wo, mat, lane_smp);
-        if (e.valid()) {
-          float rev_pdf = bsdf_reverse_pdf<SP>(sc, cam, wo, mat, lane_smp);
-          V3 c_value = spec_to_rgb<SP>(sc, e.func * Spec<SP>::make3(bqc), cam.wavelength);
-          float w_light = dvcm * vc_weight + nd.w * e.pdf;
-          float w_camera = b_wcam_base + b_dvm * rev_pdf;
-          float weight = use_mis ? (1.0f / (1.0f + w_light + w_camera)) : 1.0f;
-          float kernel_weight = use_epan ? fmaxf(2.0f * (1.0f - distance_squared * g.inv_radius_squared), 0.0f) : 1.0f;
-          float kw = kernel_weight * weight;
-          atomicAdd(&s_sum[warp][s][0], c_value.x * lt.x * kw);
-          atomicAdd(&s_sum[warp][s][1], c_value.y * lt.y * kw);
-          atomicAdd(&s_sum[warp][s][2], c_value.z * lt.z * kw);
-          accepts += 1;
-        }
-      }
-    }
-  };
-
-  while (pending) {
-    uint32_t src = __ffs(pending) - 1u;
-    pending &= pending - 1u;
-    V3 bpos = shfl3(qpos, src);
-    // the eight cells (vcm_shared.hxx:895-916): lanes 0..7 fetch their ranges, then an 8-wide exclusive scan of the counts
-    uint32_t my_begin = 0, my_cnt = 0;
-    if (lane < 8u) {
-      V3 m = (bpos - g.bbox_min) / g.cell_size;
-      V3 mf = vfloor(m);
-      V3 md = m - mf;
-      int32_t acx = static_cast<int32_t>(mf.x), acy = static_cast<int32_t>(mf.y), acz = static_cast<int32_t>(mf.z);
-      int32_t cx = (lane & 1u) ? acx + ((md.x < 0.5f) ? -1 : +1) : acx;
-      int32_t cy = (lane & 2u) ? acy + ((md.y < 0.5f) ? -1 : +1) : acy;
-      int32_t cz = (lane & 4u) ? acz + ((md.z < 0.5f) ? -1 : +1) : acz;
-      uint2 r = __ldg(&g.cell_range[grid_cell_index(g.hash_table_mask, cx, cy, cz)]);
-      my_begin = r.x;
-      my_cnt = r.y - r.x;
-    }
-    uint32_t incl = my_cnt;
-#pragma unroll
-    for (uint32_t o = 1; o < 8u; o <<= 1) {
-      uint32_t v = __shfl_up_sync(kFull, incl, o);
-      if (lane >= o) incl += v;
-    }
-    uint32_t my_excl = incl - my_cnt;
-    const uint32_t total = __shfl_sync(kFull, incl, 7);
-    uint32_t e1 = __shfl_sync(kFull, my_excl, 1), e2 = __shfl_sync(kFull, my_excl, 2), e3 = __shfl_sync(kFull, my_excl, 3), e4 = __shfl_sync(kFull, my_excl, 4),
-             e5 = __shfl_sync(kFull, my_excl, 5), e6 = __shfl_sync(kFull, my_excl, 6), e7 = __shfl_sync(kFull, my_excl, 7);
-    for (uint32_t base = 0; base < total; base += 32u) {
-      uint32_t k = base + lane;
-      bool valid = k < total;
-      uint32_t c = uint32_t(k >= e1) + uint32_t(k >= e2) + uint32_t(k >= e3) + uint32_t(k >= e4) + uint32_t(k >= e5) + uint32_t(k >= e6) + uint32_t(k >= e7);
-      uint32_t cb = __shfl_sync(kFull, my_begin, c);
-      uint32_t ce = __shfl_sync(kFull, my_excl, c);
-      uint32_t j = cb + (k - ce);
-      bool inside = false;
-      float distance_squared = 0.0f, dvcm = 0.0f;
-      if (valid) {
-        float4 pd = __ldg(&g.pos_dvcm[j]);
-        V3 d = V3{pd.x, pd.y, pd.z} - bpos;
-        distance_squared = dot(d, d);
-        dvcm = pd.w;
-        inside = !(distance_squared > g.radius_squared);
-        candidates += 1;
-      }
-      uint32_t bal = __ballot_sync(kFull, inside);
-      if (inside) {
-        uint32_t slot = n_list + __popc(bal & lane_lt);
-        s_idx[warp][slot] = j;
-        s_d2[warp][slot] = distance_squared;
-        s_dvcm[warp][slot] = dvcm;
-        s_src[warp][slot] = src;
-      }
-      n_list += __popc(bal);
-      __syncwarp();
-      if (n_list >= 32u) {
-        finish(32u);
-        __syncwarp();
-        uint32_t rest = n_list - 32u;  // < 32: move the tail to the front
-        uint32_t tj = 0, ts = 0;
-        float td = 0.0f, tv = 0.0f;
-        if (lane < rest) {
-          tj = s_idx[warp][32u + lane];
-          td = s_d2[warp][32u + lane];
-          tv = s_dvcm[warp][32u + lane];
-          ts = s_src[warp][32u + lane];
-        }
-        __syncwarp();
-        if (lane < rest) {
-          s_idx[warp][lane] = tj;
-          s_d2[warp][lane] = td;
-          s_dvcm[warp][lane] = tv;
-          s_src[warp][lane] = ts;
-        }
-        n_list = rest;
-        __syncwarp();
-      }
-    }
-  }
-  if (n_list) finish(n_list);
-  __syncwarp();
-  if (merge_queries) {
-    V3 l = {s_sum[warp][lane][0], s_sum[warp][lane][1], s_sum[warp][lane][2]};
-    if (SP) l *= V3{0.817660332f, 1.05418909f, 1.09945524f};  // kRGBLuminanceScale (:876-878)
-    float4 mg = p.paths.merged[i];
-    p.paths.merged[i] = make_float4(mg.x + l.x, mg.y + l.y, mg.z + l.z, 0.0f);
-  }
-  counter_add(&p.counters->merge_queries, merge_queries);
-  counter_add(&p.counters->merge_candidates, candidates);
-  counter_add(&p.counters->merge_accepts, accepts);
-}
-
-// Product build, scenes with stochastic BSDFs: the generic gather on vertex closures (dclosure.cuh).  Same structure as the batched kernel
-// above — the (query, photon) pairs of a warp's queries go through one shared list, 32 pairs per step whatever query they belong to — but the
-// camera vertex of a query is PREPARED once (material record -> evaluated IORs, thin film, roughness, tints: a Closure in shared memory)
-// instead of being re-derived from the Material inside every evaluate / pdf call of every pair, and one closure_evaluate returns value,
-// pdf and reverse pdf together.  Same pairs and per-pair sampler streams (path seed x photon index) as the batched kernel.
+// Product build, scenes with stochastic BSDFs: the generic gather on vertex closures (dclosure.cuh).  The evaluations are batched ACROSS
+// the queries of a warp: the (query, photon) pairs of all its queries go through one shared list, 32 pairs per step whatever query they
+// belong to, and the contributions meet in per-query shared accumulators.  The camera vertex of a query is PREPARED once (material record ->
+// evaluated IORs, thin film, roughness, tints: a Closure in shared memory) instead of being re-derived from the Material inside every
+// evaluate / pdf call of every pair, and one closure_evaluate returns value, pdf and reverse pdf together.  Each in-radius photon is
+// evaluated with a lane-local sampler derived from (path seed, photon index) and the path's sampler advances by one draw per query —
+// statistically equivalent to the reference's serial order (which the parity build keeps), 32x more parallel.
 constexpr uint32_t kClosureWarpsPerBlock = 4;
-#ifndef ETXB_CLOSURE_MIN_BLOCKS
-#define ETXB_CLOSURE_MIN_BLOCKS 4
-#endif
+constexpr int kClosureMinBlocks = 4;
 struct MergeQueryAux {
   float qc[3];  // t_camera = throughput / pdf(lambda)
   float wcam_base, dvm;
   uint32_t depth, seed;
 };
 template <bool SP>
-__global__ void __launch_bounds__(kClosureWarpsPerBlock * 32, ETXB_CLOSURE_MIN_BLOCKS) k_camera_merge_closure(const __grid_constant__ LaunchParams p, const uint32_t* sorted_ids, const uint32_t* sorted_keys, const uint32_t* count_in,
+__global__ void __launch_bounds__(kClosureWarpsPerBlock * 32, kClosureMinBlocks) k_camera_merge_closure(const __grid_constant__ LaunchParams p, const uint32_t* sorted_ids, const uint32_t* sorted_keys, const uint32_t* count_in,
                                                                                      uint32_t queries_per_warp) {
   __shared__ Closure<SP> s_cl[kClosureWarpsPerBlock][32];
   __shared__ MergeQueryAux s_aux[kClosureWarpsPerBlock][32];
@@ -1729,200 +1426,8 @@ __global__ void __launch_bounds__(kClosureWarpsPerBlock * 32, ETXB_CLOSURE_MIN_B
   counter_add(&p.counters->merge_accepts, accepts);
 }
 
-// EXPERIMENT (ETXB_MERGE_TILED=1, default off: written after the round's GPU budget ended, not yet run on the device).
-// Cell-tiled Lambert gather.  k_camera_merge_coop<SP, false> re-reads the ~530 candidate positions of a query's eight cells from L2 for every
-// query, although the 32 queries of a warp (sorted by base cell) share almost all of them: measured, the sweep streams ~3.9 TB/s out of L2.
-// Here the lanes ARE the queries: for every distinct base cell among the warp's queries, each of the up-to-27 neighbouring cells some lane
-// needs is read ONCE (coalesced, 32 photons per step), each photon is broadcast by shuffle and tested by every lane that has that cell
-// among its eight (same hash entries, same duplicates as VCMSpatialGridData::gather, vcm_shared.hxx:886-924); accepted (query, photon)
-// pairs go through the shared list and per-query accumulators of the batched generic kernel.  Candidate traffic per warp: ~29 KB instead
-// of ~270 KB.
-template <bool SP>
-__global__ void __launch_bounds__(kMergeWarpsPerBlock * 32) k_camera_merge_tiled(const __grid_constant__ LaunchParams p, const uint32_t* sorted_ids, const uint32_t* sorted_keys, const uint32_t* count_in,
-                                                                                 uint32_t queries_per_warp) {
-  __shared__ uint32_t s_idx[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_d2[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_dvcm[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ uint32_t s_src[kMergeWarpsPerBlock][kMergeListSize];
-  __shared__ float s_sum[kMergeWarpsPerBlock][32][3];
-  constexpr uint32_t kFull = 0xffffffffu;
-  const DeviceScene& sc = p.scene;
-  const GridData& g = p.grid;
-  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  const uint32_t lane_lt = (1u << lane) - 1u;
-  uint32_t q = ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * queries_per_warp + lane;
-  uint32_t merge_queries = 0, candidates = 0, accepts = 0;
-  bool active = (lane < queries_per_warp) && (q < *count_in) && (sorted_keys[q] != 0xffffffffu);
-  uint32_t i = 0;
-  V3 qpos = {0, 0, 0}, qnrm = {0, 0, 0}, qfn = {0, 0, 0}, qc = {0, 0, 0};
-  float q_wcam_base = 0.0f, q_dvm = 0.0f, q_rev_cos = 0.0f;
-  uint32_t q_depth = 0;
-  int32_t acx = 0, acy = 0, acz = 0, sx = 0, sy = 0, sz = 0;  // base cell and the side of it the query lies on (vcm_shared.hxx:895-905)
-  if (active) {
-    i = sorted_ids[q];
-    float4 hit = p.paths.hit[i];
-    PathState<SP> state = load_state<SP>(p.paths, i);
-    Isect isect = stage_intersection<SP>(p, state, i, hit);
-    const etxb_material& mat = sc.materials[isect.material_index];
-    active = merge_is_lambert(mat);
-    if (active) {
-      merge_queries = 1;
-      qpos = isect.pos;
-      qnrm = isect.nrm;
-      q_wcam_base = state.d_vcm * p.vcm.vc_weight;
-      q_dvm = state.d_vm;
-      q_depth = state.total_path_depth;
-      Spec<SP> t_camera = state.throughput / sampling_pdf<SP>(state.wavelength);
-      bool entering = dot(isect.nrm, isect.w_i) < 0.0f;
-      qfn = entering ? isect.nrm : -isect.nrm;
-      Spec<SP> diffuse = apply_image<SP>(sc, mat.scattering, isect.tex, state.wavelength);
-      qc = spec_to_rgb<SP>(sc, (diffuse / kPi) * t_camera, state.wavelength);
-      q_rev_cos = dot(isect.nrm, -isect.w_i);
-      V3 m = (qpos - g.bbox_min) / g.cell_size;
-      V3 mf = vfloor(m);
-      V3 md = m - mf;
-      acx = static_cast<int32_t>(mf.x);
-      acy = static_cast<int32_t>(mf.y);
-      acz = static_cast<int32_t>(mf.z);
-      sx = (md.x < 0.5f) ? -1 : +1;
-      sy = (md.y < 0.5f) ? -1 : +1;
-      sz = (md.z < 0.5f) ? -1 : +1;
-    }
-  }
-  s_sum[warp][lane][0] = 0.0f;
-  s_sum[warp][lane][1] = 0.0f;
-  s_sum[warp][lane][2] = 0.0f;
-  __syncwarp();
-  const bool use_mis = p.vcm.enable_mis();
-  const bool use_epan = (p.vcm.kernel == 1u);
-  const float vc_weight = p.vcm.vc_weight;
-  uint32_t n_list = 0;
-
-  auto shfl3 = [&](V3 v, uint32_t s) { return V3{__shfl_sync(kFull, v.x, s), __shfl_sync(kFull, v.y, s), __shfl_sync(kFull, v.z, s)}; };
-  auto finish = [&](uint32_t n) {
-    uint32_t j = 0, s = 0;
-    float distance_squared = 0.0f, dvcm = 0.0f;
-    if (lane < n) {
-      j = s_idx[warp][lane];
-      distance_squared = s_d2[warp][lane];
-      dvcm = s_dvcm[warp][lane];
-      s = s_src[warp][lane];
-    }
-    V3 bnrm = shfl3(qnrm, s), bfn = shfl3(qfn, s);
-    float b_wcam_base = __shfl_sync(kFull, q_wcam_base, s);
-    float b_dvm = __shfl_sync(kFull, q_dvm, s);
-    float b_rev_cos = __shfl_sync(kFull, q_rev_cos, s);
-    uint32_t b_depth = __shfl_sync(kFull, q_depth, s);
-    if (lane < n) {
-      float4 wl = __ldg(&g.win_len[j]);
-      float4 nd = __ldg(&g.nrm_dvm[j]);
-      float4 lt = __ldg(&g.thr_rgb[j]);
-      bool ok = !(__float_as_uint(wl.w) + b_depth + 1 > sc.max_path_length);
-      ok = ok && !(dot(bnrm, V3{nd.x, nd.y, nd.z}) <= kEpsilon);
-      float cos_o = -(bfn.x * wl.x + bfn.y * wl.y + bfn.z * wl.z);  // local_w_o.z of DiffuseBSDF::evaluate(-w_in)
-      ok = ok && (cos_o > kEpsilon);
-      if (ok) {
-        float bsdf_pdf_v = kInvPi * cos_o;
-        float facing = (dot(bnrm, V3{wl.x, wl.y, wl.z}) < 0.0f) ? b_rev_cos : -b_rev_cos;
-        float rev_pdf = (facing <= kEpsilon) ? 0.0f : kInvPi * facing;
-        float w_light = dvcm * vc_weight + nd.w * bsdf_pdf_v;
-        float w_camera = b_wcam_base + b_dvm * rev_pdf;
-        float weight = use_mis ? (1.0f / (1.0f + w_light + w_camera)) : 1.0f;
-        float kernel_weight = use_epan ? fmaxf(2.0f * (1.0f - distance_squared * g.inv_radius_squared), 0.0f) : 1.0f;
-        float kw = kernel_weight * weight;
-        atomicAdd(&s_sum[warp][s][0], lt.x * kw);
-        atomicAdd(&s_sum[warp][s][1], lt.y * kw);
-        atomicAdd(&s_sum[warp][s][2], lt.z * kw);
-        accepts += 1;
-      }
-    }
-  };
-
-  uint32_t todo = __ballot_sync(kFull, active);
-  while (todo) {
-    // one group = the queries of this warp that share a base cell
-    const uint32_t leader = __ffs(todo) - 1u;
-    const int32_t bx = __shfl_sync(kFull, acx, leader), by = __shfl_sync(kFull, acy, leader), bz = __shfl_sync(kFull, acz, leader);
-    const bool in_group = active && (acx == bx) && (acy == by) && (acz == bz);
-    todo &= ~__ballot_sync(kFull, in_group);
-#pragma unroll 1
-    for (int32_t o = 0; o < 27; ++o) {
-      const int32_t ox = (o % 3) - 1, oy = ((o / 3) % 3) - 1, oz = (o / 9) - 1;
-      // a query's eight cells: base or the neighbour on its side, per axis
-      const bool need = in_group && ((ox == 0) || (ox == sx)) && ((oy == 0) || (oy == sy)) && ((oz == 0) || (oz == sz));
-      if (__ballot_sync(kFull, need) == 0u) continue;
-      const uint2 range = __ldg(&g.cell_range[grid_cell_index(g.hash_table_mask, bx + ox, by + oy, bz + oz)]);
-      for (uint32_t base = range.x; base < range.y; base += 32u) {
-        const uint32_t chunk = umin(32u, range.y - base);
-        float4 pd = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-        if (lane < chunk) pd = __ldg(&g.pos_dvcm[base + lane]);
-        for (uint32_t t = 0; t < chunk; ++t) {
-          const float px = __shfl_sync(kFull, pd.x, t), py = __shfl_sync(kFull, pd.y, t), pz = __shfl_sync(kFull, pd.z, t), pw = __shfl_sync(kFull, pd.w, t);
-          bool inside = false;
-          float distance_squared = 0.0f;
-          if (need) {
-            V3 d = V3{px, py, pz} - qpos;
-            distance_squared = dot(d, d);
-            inside = !(distance_squared > g.radius_squared);
-            candidates += 1;
-          }
-          const uint32_t bal = __ballot_sync(kFull, inside);
-          if (bal == 0u) continue;
-          if (inside) {
-            uint32_t slot = n_list + __popc(bal & lane_lt);
-            s_idx[warp][slot] = base + t;
-            s_d2[warp][slot] = distance_squared;
-            s_dvcm[warp][slot] = pw;
-            s_src[warp][slot] = lane;
-          }
-          n_list += __popc(bal);
-          __syncwarp();
-          if (n_list >= 32u) {
-            finish(32u);
-            __syncwarp();
-            uint32_t rest = n_list - 32u;  // < 32: move the tail to the front
-            uint32_t tj = 0, ts = 0;
-            float td = 0.0f, tv = 0.0f;
-            if (lane < rest) {
-              tj = s_idx[warp][32u + lane];
-              td = s_d2[warp][32u + lane];
-              tv = s_dvcm[warp][32u + lane];
-              ts = s_src[warp][32u + lane];
-            }
-            __syncwarp();
-            if (lane < rest) {
-              s_idx[warp][lane] = tj;
-              s_d2[warp][lane] = td;
-              s_dvcm[warp][lane] = tv;
-              s_src[warp][lane] = ts;
-            }
-            n_list = rest;
-            __syncwarp();
-          }
-        }
-      }
-    }
-  }
-  if (n_list) finish(n_list);
-  __syncwarp();
-  if (merge_queries) {
-    V3 l = {s_sum[warp][lane][0], s_sum[warp][lane][1], s_sum[warp][lane][2]};
-    if (SP) l *= V3{0.817660332f, 1.05418909f, 1.09945524f};  // kRGBLuminanceScale (:876-878)
-    l = qc * l;
-    float4 mg = p.paths.merged[i];
-    p.paths.merged[i] = make_float4(mg.x + l.x, mg.y + l.y, mg.z + l.z, 0.0f);
-  }
-  counter_add(&p.counters->merge_queries, merge_queries);
-  counter_add(&p.counters->merge_candidates, candidates);
-  counter_add(&p.counters->merge_accepts, accepts);
-}
-
-// One CTA of kTraversalBlock threads per SM: the staged nodelet then costs 32 KB of the SM's shared memory / L1 once (four 256-thread CTAs each
-// staging their own copy took 128 KB away from the L1 that caches the rest of the tree: ncu, L1 hit rate 64 % -> 46 %, and the kernel got slower).
-constexpr uint32_t kTraversalBlock = 1024u;
-
-// Closest hit for every queued path (Raytracing::trace, rt.cxx:428-466) on persistent warps with the top of the BVH in shared memory and lane
-// refill (dtrav.cuh).  Same per-ray walk, candidate order and sampler draws as k_trace_closest / the oracle.
+// Candidate test of the closest-hit walk (Raytracing::trace, rt.cxx:428-466): Void surfaces and alpha-rejected hits are skipped, any other
+// candidate becomes the closest hit so far.
 struct ClosestHitVisitor {
   const DeviceScene& sc;
   Smp* smp;
@@ -1935,65 +1440,13 @@ struct ClosestHitVisitor {
     return kCandAccept;
   }
 };
-__global__ void __launch_bounds__(kTraversalBlock) k_trace_closest_persistent(const __grid_constant__ LaunchParams p, const uint32_t* queue, const uint32_t* queue_count, uint32_t* material_keys,
-                                                                  uint32_t key_limit, uint32_t* cursor) {
-  __shared__ __align__(128) BvhNode s_nodes[kNodeletNodes];
-  __shared__ __align__(8) uint64_t s_bar;
-  const uint32_t staged = nodelet_stage(s_nodes, &s_bar, p.scene.bvh_nodes, p.scene.bvh_node_count);
-  const StagedNodes nodes{s_nodes, p.scene.bvh_nodes, staged};
-  const uint32_t total = *queue_count;
-  // the host sorts `key_limit` (its upper bound of the queue size) slots by material: slots past the device-side count sort last
-  if (material_keys != nullptr) {
-    for (uint32_t q = total + blockIdx.x * blockDim.x + threadIdx.x; q < key_limit; q += gridDim.x * blockDim.x) material_keys[q] = queue_key_past_count(p);
-  }
-  bool active = false, exhausted = false;
-  uint32_t q = 0, i = 0, n_nodes = 0, n_tris = 0, rays = 0;
-  RayWalk walk;
-  int32_t stack[kBvhStackSize];
-  Smp smp;
-  smp.seed = 0;
-  smp.fixed_u = smp.fixed_v = smp.fixed_w = 0.0f;
-  HitRec best = {0.0f, 0.0f, 0.0f, kInvalidIndex};
-  ClosestHitVisitor visit{p.scene, &smp, &best};
-  for (;;) {
-    uint32_t next = 0;
-    if (warp_refill(!active, cursor, total, next, exhausted)) {
-      q = next;
-      i = queue[q];
-      float4 o = p.paths.ray_o[i], d = p.paths.ray_d[i];
-      smp.seed = p.paths.misc[i].x;
-      best = {0.0f, 0.0f, 0.0f, kInvalidIndex};
-      walk.begin({o.x, o.y, o.z}, {d.x, d.y, d.z}, o.w, d.w);
-      active = true;
-      rays += 1u;
-    }
-    if (!__any_sync(0xffffffffu, active)) break;
-    while (active) {
-      if (walk_step(walk, stack, nodes, p.scene.bvh_tris, visit, n_nodes, n_tris)) {
-        p.paths.hit[i] = make_float4(best.u, best.v, best.t, __uint_as_float(best.tri));
-        p.paths.misc[i].x = smp.seed;
-        if (material_keys != nullptr) material_keys[q] = queue_sort_key(p, best.tri, p.paths.ray_o[i], p.paths.ray_d[i], best.t);
-        active = false;
-      } else if (!exhausted && (__popc(__activemask()) < kRefillLanes)) {
-        break;  // too few lanes left in this walk: go and fetch rays for the idle ones
-      }
-    }
-  }
-  counter_add(&p.counters->rays_closest, rays);
-#ifdef ETXB_COUNT_TRAVERSAL
-  counter_add(&p.counters->nodes, n_nodes);
-  counter_add(&p.counters->tris, n_tris);
-  counter_add(&p.counters->nodes_closest, n_nodes);
-  counter_add(&p.counters->tris_closest, n_tris);
-#endif
-}
 
 // Closest hit through the 4-wide quantised tree (dwide.cuh), one ray per thread: the product build's kernel for scenes with stochastic BSDFs.
 __global__ void __launch_bounds__(256) k_trace_closest_wide(const __grid_constant__ LaunchParams p, const uint32_t* queue, const uint32_t* queue_count, uint32_t* material_keys,
                                                             uint32_t key_limit) {
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= *queue_count) {
-    if ((material_keys != nullptr) && (q < key_limit)) material_keys[q] = queue_key_past_count(p);
+    if ((material_keys != nullptr) && (q < key_limit)) material_keys[q] = kQueueKeyPastCount;
     return;
   }
   uint32_t i = queue[q];
@@ -2012,7 +1465,7 @@ __global__ void __launch_bounds__(256) k_trace_closest_wide(const __grid_constan
   }
   p.paths.hit[i] = make_float4(best.u, best.v, best.t, __uint_as_float(best.tri));
   p.paths.misc[i].x = smp.seed;
-  if (material_keys != nullptr) material_keys[q] = queue_sort_key(p, best.tri, o, d, best.t);
+  if (material_keys != nullptr) material_keys[q] = queue_sort_key(p, best.tri);
   counter_add(&p.counters->rays_closest, 1u);
 #ifdef ETXB_COUNT_TRAVERSAL
   counter_add(&p.counters->nodes, n_nodes);
@@ -2022,33 +1475,15 @@ __global__ void __launch_bounds__(256) k_trace_closest_wide(const __grid_constan
 #endif
 }
 
-// The shadow segments of one bounce (ShadowBatch, atomic mode): any-hit on the same persistent, nodelet-staged, lane-refilled walk; a segment
+// One CTA of kTraversalBlock threads per SM: the staged nodelet then costs 32 KB of the SM's shared memory / L1 once (four 256-thread CTAs each
+// staging their own copy took 128 KB away from the L1 that caches the rest of the tree: ncu, L1 hit rate 64 % -> 46 %, and the kernel got slower).
+constexpr uint32_t kTraversalBlock = 1024u;
+
+// The shadow segments of one bounce (ShadowBatch, atomic mode): any-hit on a persistent, nodelet-staged, lane-refilled walk (dtrav.cuh); a segment
 // that reaches its end adds its contribution to its target (a path's gathered sum, or a pixel of the light image).  Opaque scenes only: any
 // non-Void surface on the segment occludes (rt.cxx:468-579 without Boundary crossings).
-// Experiment (ETXB_SHADOW_SORT=1, default off): order of the bounce's shadow list by the Morton code of the segments' origins, so that the rays a warp
-// of k_shadow_resolve walks together start in the same region of the tree.  keys[i] for the `upper` slots the host sorts (its upper bound of the
-// device-side count): 30-bit Morton code inside the scene's bounding cube, 0xffffffff past the count; vals[i] = i.
-__global__ void __launch_bounds__(256) k_shadow_keys(const __grid_constant__ LaunchParams p, uint32_t upper, uint32_t* keys, uint32_t* vals) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= upper) return;
-  const uint32_t count = umin(p.shadow_count[0], p.shadow_capacity);
-  uint32_t key = 0xffffffffu;
-  if (i < count) {
-    float4 a = p.shadow_p0[i];
-    const float r = p.scene.bounding_sphere_radius;
-    const V3 c = p.scene.bounding_sphere_center;
-    const float scale = 1024.0f / fmaxf(2.0f * r, 1e-20f);
-    uint32_t x = umin(uint32_t(fmaxf((a.x - (c.x - r)) * scale, 0.0f)), 1023u);
-    uint32_t y = umin(uint32_t(fmaxf((a.y - (c.y - r)) * scale, 0.0f)), 1023u);
-    uint32_t z = umin(uint32_t(fmaxf((a.z - (c.z - r)) * scale, 0.0f)), 1023u);
-    key = morton_part(x) | (morton_part(y) << 1) | (morton_part(z) << 2);
-  }
-  keys[i] = key;
-  vals[i] = i;
-}
-
 template <bool WIDE>
-__global__ void __launch_bounds__(kTraversalBlock) k_shadow_resolve(const __grid_constant__ LaunchParams p, uint32_t* cursor, const uint32_t* order) {
+__global__ void __launch_bounds__(kTraversalBlock) k_shadow_resolve(const __grid_constant__ LaunchParams p, uint32_t* cursor) {
   // 32 KB of shared memory: the top kNodeletNodes nodes of the tree this instantiation walks (both node types are 64 bytes)
   __shared__ __align__(128) BvhNode s_nodes[kNodeletNodes];
   __shared__ __align__(8) uint64_t s_bar;
@@ -2083,7 +1518,7 @@ __global__ void __launch_bounds__(kTraversalBlock) k_shadow_resolve(const __grid
   for (;;) {
     uint32_t next = 0;
     if (warp_refill(!active, cursor, total, next, exhausted)) {
-      k = (order != nullptr) ? order[next] : next;
+      k = next;
       float4 a = p.shadow_p0[k], b = p.shadow_p1[k];
       target = reinterpret_cast<const uint32_t*>(p.shadow_p1 + k)[3];  // raw bits (see ShadowBatch::push_rgb)
       V3 direction = V3{b.x, b.y, b.z} - V3{a.x, a.y, a.z};

@@ -94,7 +94,7 @@ __global__ void __launch_bounds__(128) k_pt_begin(const __grid_constant__ Launch
 // run_path_iteration after the trace (:485-510): medium event, surface hit or miss.  A path that goes on is queued for the next bounce; one that
 // ends leaves its sums in the path columns for k_pt_accumulate.
 template <bool SP, bool PLAIN>
-__global__ void __launch_bounds__(128, ETXB_BOUNCE_MIN_BLOCKS) k_pt_shade(const __grid_constant__ LaunchParams p, const __grid_constant__ PtParams pt, const uint32_t* queue_in,
+__global__ void __launch_bounds__(128, kBounceMinBlocks) k_pt_shade(const __grid_constant__ LaunchParams p, const __grid_constant__ PtParams pt, const uint32_t* queue_in,
                                                                            const uint32_t* count_in, uint32_t* queue_out, uint32_t* count_out) {
   uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
   uint32_t shadow_rays = 0, i = 0;

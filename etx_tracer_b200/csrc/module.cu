@@ -102,23 +102,8 @@ struct etxb_ctx {
   bool spectral = false;
   bool profile = false;
   bool has_stochastic_merge = false;  // some material that can be merged at is not Lambert (needs the serial gather)
-  bool merge_tiled = false;           // experiment, default off: cell-tiled Lambert gather k_camera_merge_tiled (ETXB_MERGE_TILED=1)
-  bool merge_material_major = true;   // gather queue ordered by (material, Morton code): the warps in flight evaluate one BSDF class at a time (measured on the B200,
-                                      // round 2: C3 generic gather 60.6 -> 46.1 ms per iteration; ETXB_MERGE_MATERIAL_MAJOR=0 switches it off)
-  bool plain_kernels = true;          // bounce kernels specialised for scenes without media / Boundary surfaces / subsurface (ETXB_PLAIN_KERNELS=0: general ones)
-  bool plain_scene = false;           // set at upload: the scene qualifies
+  bool plain_scene = false;           // set at upload: no media / Boundary surfaces / subsurface, so the bounce kernels take their specialised instantiation
   bool opaque_scene = false;          // set at upload: no alpha test can reject a hit (every opacity 1, no alpha images), no Boundary surfaces / media
-  bool shadow_atomic = true;          // product build, opaque scenes with stochastic BSDFs: shadow segments resolved by k_shadow_resolve (ETXB_SHADOW_ATOMIC=0: inline)
-  bool queue_sort_spatial = false;    // experiment (ETXB_QUEUE_SORT_SPATIAL=1): path queues sorted by (hit material, Morton code of the hit point)
-  bool shadow_sort = false;           // experiment (ETXB_SHADOW_SORT=1): long shadow lists are walked in the Morton order of the segments' origins
-  bool persistent_trace = false;      // closest hits on the persistent, nodelet-staged, lane-refilled kernel (ETXB_TRACE_PERSISTENT=1).  Measured on the B200 (C3,
-                                      // round 2): 27.1 ms per iteration against 22.9 ms for the thread-per-ray kernel — one ray per path leaves little to refill
-                                      // from, and the walk's dynamic stack costs the same either way — so the default stays thread-per-ray; the shadow segments
-                                      // (2-3x as many rays, from one list) always go through the persistent kernel
-  bool merge_closure = true;          // generic photon gather on vertex closures (dclosure.cuh; ETXB_MERGE_CLOSURE=0: the batched generic kernel of round 1)
-  bool merge_batched = true;          // generic photon gather batches its BSDF evaluations across the queries of a warp (ETXB_MERGE_BATCHED=0: per query)
-  bool sort_by_material = true;       // group path queues and the connection list by material where BSDFs are costly (ETXB_SORT_MATERIAL=0: A/B switch)
-  bool connect_deferred = true;       // per-connection stage for scenes with deferred shadow rays (ETXB_CONNECT_DEFERRED=0: A/B switch, serial loop)
 
   // scene in HBM
   DevBuf<DVertex> vertices;
@@ -136,7 +121,6 @@ struct etxb_ctx {
   DevBuf<BvhNode> bvh_nodes;
   DevBuf<WideNode> wide_nodes;
   bool debug_trace_wide = false;      // etxb_debug_select_tree: etxb_debug_trace walks the 4-wide tree when the scene has one
-  bool wide_bvh = true;               // product build, scenes with stochastic BSDFs: closest hits and shadow segments walk the 4-wide quantised tree (ETXB_WIDE_BVH=0: BVH2)
   DevBuf<float4> bvh_tris;
   DevBuf<float> xyz_table, rgb_response_table;
   DevBuf<uint8_t> bn_sobol, bn_scrambling, bn_ranking;
@@ -372,7 +356,7 @@ LaunchParams make_params(etxb_ctx* ctx) {
   p.conn_list = ctx->conn_list.ptr;
   p.conn_count = ctx->conn_count.ptr;
   p.conn_capacity = ctx->lv_capacity;
-  p.conn_key = (ctx->sort_by_material && ctx->has_stochastic_merge && ctx->conn_list_sorted.count) ? ctx->keys_in.ptr : nullptr;  // keys_in / vals_in are free after the grid build
+  p.conn_key = (ctx->has_stochastic_merge && ctx->conn_list_sorted.count) ? ctx->keys_in.ptr : nullptr;  // keys_in / vals_in are free after the grid build
   p.paths.shadow_span = ctx->shadow_span.ptr;
   p.shadow_p0 = ctx->shadow_p0.ptr;
   p.shadow_p1 = ctx->shadow_p1.ptr;
@@ -381,15 +365,12 @@ LaunchParams make_params(etxb_ctx* ctx) {
   p.shadow_count = ctx->shadow_count.ptr;
   p.shadow_capacity = uint32_t(ctx->shadow_p0.count);
   p.shadow_stage = (ctx->dscene.deferred_shadow_rays && ctx->shadow_p0.count) ? 1u : 0u;
-  p.connect_deferred = (p.shadow_stage && ctx->connect_deferred) ? 1u : 0u;
 #if defined(ETXB_PARITY) && ETXB_PARITY
   p.shadow_atomic = 0;
 #else
-  p.shadow_atomic = (ctx->shadow_atomic && !p.shadow_stage && ctx->opaque_scene && ctx->plain_scene && ctx->plain_kernels && ctx->has_stochastic_merge && ctx->shadow_p0.count) ? 1u : 0u;
+  p.shadow_atomic = (!p.shadow_stage && ctx->opaque_scene && ctx->plain_scene && ctx->has_stochastic_merge && ctx->shadow_p0.count) ? 1u : 0u;
 #endif
-  p.closures = ctx->merge_closure ? 1u : 0u;
-  p.merge_material_major = (ctx->merge_material_major && ctx->has_stochastic_merge) ? 1u : 0u;
-  p.spatial_keys = ctx->queue_sort_spatial ? 1u : 0u;
+  p.merge_material_major = ctx->has_stochastic_merge ? 1u : 0u;
 #if defined(ETXB_PARITY) && ETXB_PARITY
   p.connect_stage = 0;
 #else
@@ -444,47 +425,32 @@ int next_queue_size(etxb_ctx* ctx, const uint32_t* dptr, uint32_t& active, uint3
 // past the device-side count); a stable 9-bit radix sort groups the queue, slots past the count stay at the end.  Returns the queue the
 // rest of the bounce must use.  Short queues (the tail of a pass) are latency bound and skip it.
 constexpr uint32_t kSortQueueMin = 1024u;
-inline bool sorts_queue(const etxb_ctx* ctx, uint32_t active) { return ctx->sort_by_material && ctx->has_stochastic_merge && (active >= kSortQueueMin) && ctx->queue_sorted.count; }
+inline bool sorts_queue(const etxb_ctx* ctx, uint32_t active) { return ctx->has_stochastic_merge && (active >= kSortQueueMin) && ctx->queue_sorted.count; }
 int sort_queue_by_material(etxb_ctx* ctx, const uint32_t* queue, uint32_t active, const uint32_t** sorted) {
   size_t temp_bytes = ctx->cub_temp.bytes();
-  CUDA_OK(ctx, cub::DeviceRadixSort::SortPairs(ctx->cub_temp.ptr, temp_bytes, ctx->queue_keys.ptr, ctx->queue_keys_sorted.ptr, queue, ctx->queue_sorted.ptr, int(active), 0,
-                 ctx->queue_sort_spatial ? 32 : 9, ctx->stream));
+  CUDA_OK(ctx, cub::DeviceRadixSort::SortPairs(ctx->cub_temp.ptr, temp_bytes, ctx->queue_keys.ptr, ctx->queue_keys_sorted.ptr, queue, ctx->queue_sorted.ptr, int(active), 0, 9,
+                 ctx->stream));
   *sorted = ctx->queue_sorted.ptr;
   return ETXB_OK;
 }
 
-// closest hits of a queue: persistent, nodelet-staged, lane-refilled walk (dtrav.cuh) or the thread-per-ray kernel (A/B switch)
-int launch_trace_closest(etxb_ctx* ctx, const LaunchParams& p, const uint32_t* queue, const uint32_t* count, uint32_t* keys, uint32_t active) {
-  if (ctx->persistent_trace) {
-    CUDA_OK(ctx, cudaMemsetAsync(ctx->trace_cursor.ptr, 0, 4, ctx->stream));
-    const uint32_t blocks = std::min<uint32_t>(blocks_for(active, kTraversalBlock), 148u);
-    k_trace_closest_persistent<<<blocks, kTraversalBlock, 0, ctx->stream>>>(p, queue, count, keys, active, ctx->trace_cursor.ptr);
-  } else if (p.scene.wide_nodes != nullptr) {
+// closest hits of a queue, one ray per thread.  The persistent, nodelet-staged, lane-refilled walk that the shadow segments take (2-3x as many
+// rays, from one list) lost here on the B200 (C3, round 2: 27.1 against 22.9 ms per iteration): one ray per path leaves little to refill from.
+void launch_trace_closest(etxb_ctx* ctx, const LaunchParams& p, const uint32_t* queue, const uint32_t* count, uint32_t* keys, uint32_t active) {
+  if (p.scene.wide_nodes != nullptr) {
     k_trace_closest_wide<<<blocks_for(active, 256), 256, 0, ctx->stream>>>(p, queue, count, keys, active);
   } else {
     k_trace_closest<<<blocks_for(active, 256), 256, 0, ctx->stream>>>(p, queue, count, keys, active);
   }
-  return ETXB_OK;
 }
-// the bounce's shadow segments (ShadowBatch, atomic mode): traced and added to their targets.  seg_upper: the host's upper bound of the number of
-// segments (0: unknown) — with ETXB_SHADOW_SORT=1 a long list is walked in the Morton order of the segments' origins (experiment, default off)
-constexpr uint32_t kShadowSortMin = 1u << 16;
-int launch_shadow_resolve(etxb_ctx* ctx, const LaunchParams& p, uint32_t active, uint64_t seg_upper = 0) {
-  const uint32_t* order = nullptr;
-  if (ctx->shadow_sort && (seg_upper >= kShadowSortMin) && (seg_upper <= ctx->keys_in.count) && (seg_upper <= p.shadow_capacity)) {
-    const uint32_t upper = uint32_t(seg_upper);
-    k_shadow_keys<<<blocks_for(upper, 256), 256, 0, ctx->stream>>>(p, upper, ctx->keys_in.ptr, ctx->vals_in.ptr);
-    size_t temp_bytes = ctx->cub_temp.bytes();
-    CUDA_OK(ctx, cub::DeviceRadixSort::SortPairs(ctx->cub_temp.ptr, temp_bytes, ctx->keys_in.ptr, ctx->keys_out.ptr, ctx->vals_in.ptr, ctx->vals_out.ptr, int(upper), 0, 30, ctx->stream));
-    order = ctx->vals_out.ptr;
-    ctx->kernel_launches += 1;
-  }
-  CUDA_OK(ctx, cudaMemsetAsync(ctx->trace_cursor.ptr + 1, 0, 4, ctx->stream));
+// the bounce's shadow segments (ShadowBatch, atomic mode): traced and added to their targets
+int launch_shadow_resolve(etxb_ctx* ctx, const LaunchParams& p, uint32_t active) {
+  CUDA_OK(ctx, cudaMemsetAsync(ctx->trace_cursor.ptr, 0, 4, ctx->stream));
   const uint32_t blocks = std::min<uint32_t>(blocks_for(std::min<uint64_t>(uint64_t(active) * 4ull, 0x7fffffffull), kTraversalBlock), 148u);
   if (p.scene.wide_nodes != nullptr) {
-    k_shadow_resolve<true><<<blocks, kTraversalBlock, 0, ctx->stream>>>(p, ctx->trace_cursor.ptr + 1, order);
+    k_shadow_resolve<true><<<blocks, kTraversalBlock, 0, ctx->stream>>>(p, ctx->trace_cursor.ptr);
   } else {
-    k_shadow_resolve<false><<<blocks, kTraversalBlock, 0, ctx->stream>>>(p, ctx->trace_cursor.ptr + 1, order);
+    k_shadow_resolve<false><<<blocks, kTraversalBlock, 0, ctx->stream>>>(p, ctx->trace_cursor.ptr);
   }
   return ETXB_OK;
 }
@@ -509,7 +475,7 @@ int run_light_pass(etxb_ctx* ctx) {
     const uint32_t* q = qin;
     {
       LaunchTimer t(ctx, K_TRACE_LIGHT);
-      if (int rc = launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active)) return rc;
+      launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active);
     }
     if (sorted) {
       LaunchTimer t(ctx, K_QUEUE_SORT);
@@ -519,7 +485,7 @@ int run_light_pass(etxb_ctx* ctx) {
     if (p.shadow_atomic) CUDA_OK(ctx, cudaMemsetAsync(ctx->shadow_count.ptr, 0, 8, ctx->stream));
     {
       LaunchTimer t(ctx, K_LIGHT_BOUNCE);
-      if (ctx->plain_scene && ctx->plain_kernels) {
+      if (ctx->plain_scene) {
         k_light_bounce<SP, true><<<blocks_for(active, 128), 128, 0, ctx->stream>>>(p, q, counts + cur, qout, counts + (cur ^ 1u));
       } else {
         k_light_bounce<SP, false><<<blocks_for(active, 128), 128, 0, ctx->stream>>>(p, q, counts + cur, qout, counts + (cur ^ 1u));
@@ -528,7 +494,7 @@ int run_light_pass(etxb_ctx* ctx) {
     if (p.shadow_atomic) {
       // the light-to-camera connections of this bounce: segments -> splats (light image)
       LaunchTimer t(ctx, K_SHADOW_TRACE);
-      if (int rc = launch_shadow_resolve(ctx, p, active, active)) return rc;
+      if (int rc = launch_shadow_resolve(ctx, p, active)) return rc;
     }
     cur ^= 1u;
     std::swap(qin, qout);
@@ -648,7 +614,7 @@ int run_camera_pass(etxb_ctx* ctx) {
     const uint32_t* q = qin;  // the queue every stage of this bounce reads
     {
       LaunchTimer t(ctx, K_TRACE_CAMERA);
-      if (int rc = launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active)) return rc;
+      launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active);
     }
     if (sorted) {
       LaunchTimer t(ctx, K_QUEUE_SORT);
@@ -659,13 +625,13 @@ int run_camera_pass(etxb_ctx* ctx) {
     if (p.shadow_stage || p.shadow_atomic) CUDA_OK(ctx, cudaMemsetAsync(ctx->shadow_count.ptr, 0, 8, ctx->stream));
     {
       LaunchTimer t(ctx, K_CAMERA_SHADE);
-      if (ctx->plain_scene && ctx->plain_kernels) {
+      if (ctx->plain_scene) {
         k_camera_shade<SP, true><<<blocks_for(active, 128), 128, 0, ctx->stream>>>(p, q, counts + cur);
       } else {
         k_camera_shade<SP, false><<<blocks_for(active, 128), 128, 0, ctx->stream>>>(p, q, counts + cur);
       }
     }
-    if (p.connect_deferred && (ctx->options.options & ETXB_VCM_CONNECT_VERTICES)) {
+    if (p.shadow_stage && (ctx->options.options & ETXB_VCM_CONNECT_VERTICES)) {
       // one thread per (camera vertex, light vertex) pair of the bounce, grid-stride over the reserved shadow slots (count on the device)
       LaunchTimer t(ctx, K_CAMERA_CONNECT);
       uint32_t blocks = std::min<uint32_t>(148u * 16u, blocks_for(std::min<uint64_t>(uint64_t(active) * 8ull, 0x7fffffffull), 128));
@@ -677,13 +643,12 @@ int run_camera_pass(etxb_ctx* ctx) {
       uint32_t blocks = std::min<uint32_t>(148u * 8u, blocks_for(std::min<uint64_t>(uint64_t(active) * 32ull, 0x7fffffffull), 256));
       k_shadow_trace<<<blocks, 256, 0, ctx->stream>>>(p);
     }
-    uint64_t shadow_upper = 0;  // host-side upper bound of this bounce's shadow list (0 = not known: the tail keeps its counts on the device)
     if (p.connect_stage && (ctx->options.options & ETXB_VCM_CONNECT_VERTICES)) {
       if (active < kTailQueue) {
         // tail of the pass: the pair count stays on the device (k_camera_connect is grid-stride), no host round trip per bounce
         LaunchTimer t(ctx, K_CAMERA_CONNECT);
         const uint32_t blocks = std::min<uint32_t>(148u * 4u, blocks_for(active * 4u, 128));
-        if (ctx->plain_scene && ctx->plain_kernels) {
+        if (ctx->plain_scene) {
           k_camera_connect<SP, true><<<blocks, 128, 0, ctx->stream>>>(p, ctx->conn_list.ptr);
         } else {
           k_camera_connect<SP, false><<<blocks, 128, 0, ctx->stream>>>(p, ctx->conn_list.ptr);
@@ -692,7 +657,6 @@ int run_camera_pass(etxb_ctx* ctx) {
         uint32_t pending = 0;
         if (int rc = read_u32(ctx, ctx->conn_count.ptr, pending)) return rc;
         pending = std::min(pending, ctx->lv_capacity);
-        shadow_upper = uint64_t(pending) + active;  // one segment per vertex connection + one emitter segment per path
         if (pending) {
           const uint2* list = ctx->conn_list.ptr;
           if (p.conn_key && (pending >= kSortQueueMin)) {
@@ -704,7 +668,7 @@ int run_camera_pass(etxb_ctx* ctx) {
             list = ctx->conn_list_sorted.ptr;
           }
           LaunchTimer t(ctx, K_CAMERA_CONNECT);
-          if (ctx->plain_scene && ctx->plain_kernels) {
+          if (ctx->plain_scene) {
             k_camera_connect<SP, true><<<blocks_for(pending, 128), 128, 0, ctx->stream>>>(p, list);
           } else {
             k_camera_connect<SP, false><<<blocks_for(pending, 128), 128, 0, ctx->stream>>>(p, list);
@@ -715,7 +679,7 @@ int run_camera_pass(etxb_ctx* ctx) {
     if (p.shadow_atomic) {
       // emitter-sample and vertex-connection segments of this bounce: traced, the unoccluded ones added to their paths' gathered sums
       LaunchTimer t(ctx, K_SHADOW_TRACE);
-      if (int rc = launch_shadow_resolve(ctx, p, active, shadow_upper)) return rc;
+      if (int rc = launch_shadow_resolve(ctx, p, active)) return rc;
     }
 #if defined(ETXB_PARITY) && ETXB_PARITY
     if (merging) {
@@ -742,22 +706,12 @@ int run_camera_pass(etxb_ctx* ctx) {
       const uint32_t merge_blocks = blocks_for(blocks_for(active, qpw), kMergeWarpsPerBlock);
       {
         LaunchTimer t(ctx, K_CAMERA_MERGE);
-        if (ctx->merge_tiled) {
-          k_camera_merge_tiled<SP><<<merge_blocks, kMergeWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
-        } else {
-          k_camera_merge_coop<SP, false><<<merge_blocks, kMergeWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
-        }
+        k_camera_merge_coop<SP><<<merge_blocks, kMergeWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
       }
       if (ctx->has_stochastic_merge) {
         LaunchTimer t(ctx, K_CAMERA_MERGE_SERIAL);
-        if (ctx->merge_closure) {
-          const uint32_t closure_blocks = blocks_for(blocks_for(active, qpw), kClosureWarpsPerBlock);
-          k_camera_merge_closure<SP><<<closure_blocks, kClosureWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
-        } else if (ctx->merge_batched) {
-          k_camera_merge_generic_batched<SP><<<merge_blocks, kMergeWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
-        } else {
-          k_camera_merge_coop<SP, true><<<merge_blocks, kMergeWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
-        }
+        const uint32_t closure_blocks = blocks_for(blocks_for(active, qpw), kClosureWarpsPerBlock);
+        k_camera_merge_closure<SP><<<closure_blocks, kClosureWarpsPerBlock * 32, 0, ctx->stream>>>(p, ids, keys, counts + cur, qpw);
       }
     }
 #endif
@@ -921,8 +875,7 @@ int run_pt_iteration(etxb_ctx* ctx) {
   pt.pixel_sampler_radius = ctx->pixel_sampler_radius;
   pt.radiance_clamp = ctx->radiance_clamp;
   PtFilm pf = make_pt_film(ctx);
-  const bool plain = ctx->plain_scene && ctx->plain_kernels;
-  if (!plain) p.shadow_atomic = 0;
+  const bool plain = ctx->plain_scene;
   uint32_t* counts = ctx->queue_counts.ptr;
   CUDA_OK(ctx, cudaMemsetAsync(counts, 0, 8, ctx->stream));
   uint32_t* qin = ctx->queue_a.ptr;
@@ -940,7 +893,7 @@ int run_pt_iteration(etxb_ctx* ctx) {
     const uint32_t* q = qin;
     {
       LaunchTimer t(ctx, K_TRACE_CAMERA);
-      if (int rc = launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active)) return rc;
+      launch_trace_closest(ctx, p, qin, counts + cur, sorted ? ctx->queue_keys.ptr : nullptr, active);
     }
     if (sorted) {
       LaunchTimer t(ctx, K_QUEUE_SORT);
@@ -958,7 +911,7 @@ int run_pt_iteration(etxb_ctx* ctx) {
     }
     if (p.shadow_atomic) {
       LaunchTimer t(ctx, K_SHADOW_TRACE);
-      if (int rc = launch_shadow_resolve(ctx, p, active, active)) return rc;
+      if (int rc = launch_shadow_resolve(ctx, p, active)) return rc;
     }
     cur ^= 1u;
     std::swap(qin, qout);
@@ -1009,18 +962,6 @@ int etxb_create(etxb_ctx** out_ctx, const etxb_device_config* cfg) {
       ctx->event_pool.push_back(e);
     }
   }
-  if (const char* e = getenv("ETXB_CONNECT_DEFERRED")) ctx->connect_deferred = (e[0] != '0');
-  if (const char* e = getenv("ETXB_SORT_MATERIAL")) ctx->sort_by_material = (e[0] != '0');
-  if (const char* e = getenv("ETXB_MERGE_BATCHED")) ctx->merge_batched = (e[0] != '0');
-  if (const char* e = getenv("ETXB_MERGE_CLOSURE")) ctx->merge_closure = (e[0] != '0');
-  if (const char* e = getenv("ETXB_SHADOW_ATOMIC")) ctx->shadow_atomic = (e[0] != '0');
-  if (const char* e = getenv("ETXB_WIDE_BVH")) ctx->wide_bvh = (e[0] != '0');
-  if (const char* e = getenv("ETXB_TRACE_PERSISTENT")) ctx->persistent_trace = (e[0] != '0');
-  if (const char* e = getenv("ETXB_PLAIN_KERNELS")) ctx->plain_kernels = (e[0] != '0');
-  if (const char* e = getenv("ETXB_MERGE_MATERIAL_MAJOR")) ctx->merge_material_major = (e[0] != '0');
-  if (const char* e = getenv("ETXB_MERGE_TILED")) ctx->merge_tiled = (e[0] != '0');
-  if (const char* e = getenv("ETXB_SHADOW_SORT")) ctx->shadow_sort = (e[0] != '0');
-  if (const char* e = getenv("ETXB_QUEUE_SORT_SPATIAL")) ctx->queue_sort_spatial = (e[0] != '0');
   if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) {
     delete ctx;
     return ETXB_ERR_CUDA;
@@ -1395,7 +1336,7 @@ int etxb_upload_scene(etxb_ctx* ctx, const void* scene_blob, uint64_t scene_byte
   d.wide_nodes = nullptr;
   d.wide_node_count = 0;
 #if !(defined(ETXB_PARITY) && ETXB_PARITY)
-  if (ctx->wide_bvh && ctx->has_stochastic_merge) {
+  if (ctx->has_stochastic_merge) {
     // the sampler streams of such a scene's stochastic stages are the product build's own already: its traversal kernels may meet candidates in
     // another order, so they walk the 4-wide quantised form of the tree (dwide.cuh); Lambert / delta scenes keep the oracle's candidate order
     WideBvh wide;
@@ -1459,7 +1400,7 @@ int etxb_upload_scene(etxb_ctx* ctx, const void* scene_blob, uint64_t scene_byte
   CUDA_OK(ctx, ctx->lv_tmp.alloc(cap));
   CUDA_OK(ctx, ctx->lv_final.alloc(cap));
   CUDA_OK(ctx, ctx->conn_list.alloc(cap));
-  if (ctx->has_stochastic_merge && ctx->sort_by_material) {
+  if (ctx->has_stochastic_merge) {
     CUDA_OK(ctx, ctx->conn_list_sorted.alloc(cap));
     CUDA_OK(ctx, ctx->queue_sorted.alloc(n));
     CUDA_OK(ctx, ctx->queue_keys.alloc(n));
@@ -1470,8 +1411,8 @@ int etxb_upload_scene(etxb_ctx* ctx, const void* scene_blob, uint64_t scene_byte
     ctx->queue_keys.release();
     ctx->queue_keys_sorted.release();
   }
-  CUDA_OK(ctx, ctx->trace_cursor.alloc(4));
-  const bool atomic_candidate = ctx->shadow_atomic && ctx->opaque_scene && ctx->plain_scene && ctx->has_stochastic_merge;
+  CUDA_OK(ctx, ctx->trace_cursor.alloc(1));
+  const bool atomic_candidate = ctx->opaque_scene && ctx->plain_scene && ctx->has_stochastic_merge;
   if (ctx->dscene.deferred_shadow_rays || atomic_candidate) {
     // atomic mode: a camera bounce queues its vertex connections (<= cap, the pair list's capacity) plus one emitter segment per path
     const uint64_t shadow_cap = std::min<uint64_t>(cap + (atomic_candidate ? n : 0), 0x7fffffffull);
@@ -1489,7 +1430,7 @@ int etxb_upload_scene(etxb_ctx* ctx, const void* scene_blob, uint64_t scene_byte
     ctx->shadow_result.release();
   }
   // the sort buffers also hold the gather queue and the path queues (up to one entry per path), whatever the configured pool capacity
-  const uint64_t sort_cap = std::max<uint64_t>(cap, n) + ((ctx->shadow_sort && atomic_candidate) ? n : 0);
+  const uint64_t sort_cap = std::max<uint64_t>(cap, n);
   DevBuf<uint32_t>* per_vertex_u32[] = {&ctx->keys_in, &ctx->keys_out, &ctx->vals_in, &ctx->vals_out};
   for (auto* b : per_vertex_u32) CUDA_OK(ctx, b->alloc(sort_cap));
   DevBuf<float4>* per_vertex_f4[] = {&ctx->g_pos, &ctx->g_nrm, &ctx->g_win, &ctx->g_thr};

@@ -143,61 +143,6 @@ def test_bench_algorithmic_bytes_follow_the_survey_formula():
     assert total == sum(once.values())
 
 
-def test_cell_tiled_gather_visits_the_reference_candidate_multiset():
-    """Model of k_camera_merge_tiled's candidate generation against VCMSpatialGridData::gather (vcm_shared.hxx:886-924): for every query the
-    multiset of (photon, times visited) must be the reference's — its eight hash entries, INCLUDING the duplicates when two of the eight cells
-    collide in the hash table — although the tiled kernel walks the 27 neighbours of a base cell once per group of queries."""
-    rng = np.random.default_rng(7)
-    mask = 63  # tiny table: collisions among a query's eight cells do happen
-    cell = 0.25
-    bbox_min = np.array([-1.0, -1.0, -1.0], dtype=np.float32)
-
-    def h(x, y, z):
-        return ((np.uint32(x & 0xffffffff) * np.uint32(73856093)) ^ (np.uint32(y & 0xffffffff) * np.uint32(19349663)) ^ (np.uint32(z & 0xffffffff) * np.uint32(83492791))) & np.uint32(mask)
-
-    photons = (rng.random((600, 3), dtype=np.float32) * 2 - 1).astype(np.float32)
-    pc = np.floor((photons - bbox_min) / np.float32(cell)).astype(np.int64)
-    entry = np.array([h(int(c[0]), int(c[1]), int(c[2])) for c in pc])
-    per_entry = {e: np.nonzero(entry == e)[0] for e in range(mask + 1)}
-    queries = (rng.random((64, 3), dtype=np.float32) * 1.6 - 0.8).astype(np.float32)
-    queries[1] = queries[0] + np.float32(0.01)  # same base cell, maybe another side
-    m = (queries - bbox_min) / np.float32(cell)
-    mf = np.floor(m)
-    base = mf.astype(np.int64)
-    side = np.where((m - mf) < 0.5, -1, 1)
-
-    def reference(qi):
-        visited = []
-        for dz in (0, 1):
-            for dy in (0, 1):
-                for dx in (0, 1):
-                    c = base[qi] + np.array([dx * side[qi][0], dy * side[qi][1], dz * side[qi][2]])
-                    visited += list(per_entry[int(h(int(c[0]), int(c[1]), int(c[2])))])
-        return sorted(visited)
-
-    tiled = {qi: [] for qi in range(len(queries))}
-    for w in range(0, len(queries), 32):  # one warp = 32 queries
-        lanes = list(range(w, min(w + 32, len(queries))))
-        todo = set(lanes)
-        while todo:
-            leader = min(todo)
-            group = [qi for qi in lanes if tuple(base[qi]) == tuple(base[leader])]
-            todo -= set(group)
-            for o in range(27):
-                ox, oy, oz = (o % 3) - 1, ((o // 3) % 3) - 1, (o // 9) - 1
-                need = [qi for qi in group if (ox == 0 or ox == side[qi][0]) and (oy == 0 or oy == side[qi][1]) and (oz == 0 or oz == side[qi][2])]
-                if not need:
-                    continue
-                c = base[leader] + np.array([ox, oy, oz])
-                for j in per_entry[int(h(int(c[0]), int(c[1]), int(c[2])))]:
-                    for qi in need:
-                        tiled[qi].append(j)
-    for qi in range(len(queries)):
-        assert sorted(tiled[qi]) == reference(qi), qi
-    # the table is small enough that some query really sees a duplicate (otherwise the test would not cover that case)
-    assert any(len(reference(qi)) != len(set(reference(qi))) for qi in range(len(queries)))
-
-
 def test_replica_mode_deals_every_iteration_exactly_once():
     """etxb_group_enqueue in replica mode (module.cu replica_plan, through the device-free test hook): whole frames round-robin; with a split lane
     the n % world left-over iterations are split over world / (n % world) ranks each by camera tile.  Whatever (world, n): every ordinal is
